@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload cfg3|cfg1|cfg2_head|cfg4|cfg5_head|cfg5] [--mode bf16|fp32]
+                    [--dump-outputs DIR]
 
 One "step" = one forward+backward pass of the head over one batch of synthetic input
 (everything behind asm_forward_backward: norms, contractions, epilogues; excluding the
@@ -19,6 +20,10 @@ anything is timed (`parity` in the JSON line); a failed gate exits non-zero with
 Prints ONE JSON line on rank 0 (see the keys in main()).  `--impl reference` times the CPU
 stand-in for the reference's TensorFlow path (oracle/tf_graph_port.py; the TF code itself
 cannot run, see DESIGN.md) on the host cores for the same metric and config.
+
+`--dump-outputs DIR` writes, on rank 0, what the headline path returned from its last timed
+step as DIR/<name>.npy (see step_arrays), so that two builds run with the same arguments (hence
+the same seeded inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -42,6 +47,8 @@ LAMBDA = 5.0      # lambda_min of the SphereFace schedule (SURVEY.md 8d: timing 
 LOSS_TOL = {"fp32": 1e-5, "bf16": 2e-3}      # BASELINE.json north_star
 COS_MIN = 0.9999
 ELEM_TOL = {"fp32": 5e-5, "bf16": 2e-2}      # max |dW - oracle| / max |oracle|, every element of the checked shard
+DUMP_DW_BYTES = 32 << 20     # --dump-outputs: dW beyond this is cut to a seeded choice of class columns
+DUMP_SEED = 0
 
 
 def load_peaks():
@@ -129,13 +136,14 @@ def time_cpu_port(cfg, steps: int, warmup: int, budget_s: float):
     times = []
     for _ in range(steps):
         t = time.perf_counter()
-        port.step(X, inp.W, y, M_MARGIN, LAMBDA)
+        last = port.step(X, inp.W, y, M_MARGIN, LAMBDA)
         times.append(time.perf_counter() - t)
     total = sum(times)
     sample = (f"full workload: {steps} steps of B={Bs} rows x C={cfg['C']} classes x D={cfg['D']}, fp32, torch-CPU"
               if Bs == cfg["B"] else
               f"{steps} steps over the first {Bs} of {cfg['B']} batch rows x all C={cfg['C']} classes, fp32, torch-CPU")
-    return dict(value=Bs * steps / total, ms_per_step=1e3 * total / steps, cores=cores, sample=sample, B_sample=Bs)
+    return dict(value=Bs * steps / total, ms_per_step=1e3 * total / steps, cores=cores, sample=sample, B_sample=Bs,
+                last=last)
 
 
 def run_reference(args, cfg):
@@ -143,6 +151,8 @@ def run_reference(args, cfg):
     if rank != 0:
         return
     r = time_cpu_port(cfg, args.steps, args.warmup, budget_s=150.0)
+    if args.dump_outputs:
+        write_arrays(args.dump_outputs, step_arrays(r["last"]))
     line = {
         "impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
@@ -171,6 +181,36 @@ def _cos(a, b):
     a = np.asarray(a, dtype=np.float64).ravel()
     b = np.asarray(b, dtype=np.float64).ravel()
     return float(a @ b / max(np.sqrt((a @ a) * (b @ b)), 1e-300))
+
+
+def step_arrays(res):
+    """What a caller of a launch path receives from one step, (loss, dX, dW) with loss a tensor
+    or (cross-entropy, center loss), as float32 NumPy arrays: loss [1], center_loss [1], dX
+    [B_local, D], dW [D, C_local].  A dW larger than DUMP_DW_BYTES keeps only a fixed, seeded
+    choice of class columns (in increasing order), the same for every run of one workload."""
+    import numpy as np
+    import torch
+    loss, dX, dW = res[0], res[1], res[2]
+    out = {}
+    if isinstance(loss, tuple):
+        loss, out["center_loss"] = loss[0], loss[1].detach().float().reshape(1).cpu().numpy()
+    out["loss"] = loss.detach().float().reshape(1).cpu().numpy()
+    out["dX"] = dX.detach().float().cpu().numpy()
+    if dW is not None:
+        D, Cl = dW.shape
+        keep = DUMP_DW_BYTES // (4 * D)
+        if Cl > keep:
+            cols = np.sort(np.random.default_rng(DUMP_SEED).choice(Cl, keep, replace=False))
+            dW = dW.index_select(1, torch.from_numpy(cols).to(dW.device))
+        out["dW"] = dW.detach().float().cpu().numpy()
+    return out
+
+
+def write_arrays(directory, arrays):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------
@@ -250,6 +290,7 @@ class Workload:
         self.need_flush = Cn * D * 4 <= 126e6
         self.flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev) if self.need_flush else None
         self.paths, self.host_paths = {}, {}
+        self.outputs = {}
         self._build_paths()
 
     # ---- launch paths --------------------------------------------------------------------
@@ -406,18 +447,24 @@ class Workload:
             self.dist.barrier()
         self.torch.cuda.synchronize()
 
-    def timed(self, fn, n):
-        """n calls of fn between CUDA events on the current stream; returns ms (max over ranks)."""
+    def timed(self, fn, n, keep=None):
+        """n calls of fn between CUDA events on the current stream; returns ms (max over ranks).
+        With `keep`, what the last call returned goes to self.outputs[keep] (step_arrays)."""
         torch = self.torch
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(n):
+        for _ in range(n - 1):
             if self.flush is not None:
                 self.flush.zero_()
             fn()
+        if self.flush is not None:
+            self.flush.zero_()
+        last = fn()
         e1.record()
         self.barrier()
+        if keep is not None:
+            self.outputs[keep] = step_arrays(last)
         ms = e0.elapsed_time(e1)
         if self.world > 1:
             t = torch.tensor([ms], device=self.dev)
@@ -440,14 +487,15 @@ class Workload:
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / 20
 
-    def time_value(self, K, Wm):
-        """Device-resident timing of every launch path; the fastest is the headline."""
+    def time_value(self, K, Wm, keep_outputs=False):
+        """Device-resident timing of every launch path; the fastest is the headline.  With
+        keep_outputs, self.outputs[path] holds what each path returned from its last timed step."""
         self.flush_ms = self.flush_cost()
         value_ms = {}
         for name, fn in self.paths.items():
             for _ in range(max(Wm, 3)):
                 fn()
-            value_ms[name] = self.timed(fn, K) / K - self.flush_ms
+            value_ms[name] = self.timed(fn, K, keep=name if keep_outputs else None) / K - self.flush_ms
         best = min(value_ms, key=value_ms.get)
         return best, value_ms
 
@@ -526,7 +574,10 @@ def run_ours(args, cfg):
 
     # ---- (1) device-resident timing: the headline `value`
     t_load0 = time.time()
-    value_path, value_ms = wl.time_value(K, Wm)
+    value_path, value_ms = wl.time_value(K, Wm, keep_outputs=bool(args.dump_outputs) and rank == 0)
+    if wl.outputs:
+        write_arrays(args.dump_outputs, wl.outputs[value_path])
+        wl.outputs.clear()
     run_step = wl.paths[value_path]
     ms_step = value_ms[value_path]
     flush_ms = wl.flush_ms
@@ -534,20 +585,21 @@ def run_ours(args, cfg):
 
     # distribution of the chosen path (SURVEY 8d asks for median and p10/p90): events between
     # GROUPS of 5 steps (a timing event after every step costs ~20 us of stream serialisation,
-    # which would measure the events); the headline stays the K-step mean above
+    # which would measure the events), K steps in all; the headline stays the K-step mean above
     grp = 5 if K >= 10 else 1
-    ngrp = max(1, K // grp)
+    sizes = [grp] * (K // grp) + ([K % grp] if K % grp else [])
+    ngrp = len(sizes)
     evs = [torch.cuda.Event(enable_timing=True) for _ in range(ngrp + 1)]
     wl.barrier()
-    for gi in range(ngrp):
+    for gi, size in enumerate(sizes):
         evs[gi].record()
-        for _ in range(grp):
+        for _ in range(size):
             if wl.flush is not None:
                 wl.flush.zero_()
             run_step()
     evs[ngrp].record()
     wl.barrier()
-    per = sorted(evs[i].elapsed_time(evs[i + 1]) / grp - flush_ms for i in range(ngrp))
+    per = sorted(evs[i].elapsed_time(evs[i + 1]) / sizes[i] - flush_ms for i in range(ngrp))
     step_dist = {"p10": per[int(0.1 * (ngrp - 1))], "p50": per[(ngrp - 1) // 2],
                  "p90": per[int(round(0.9 * (ngrp - 1)))], "group": grp, "groups": ngrp,
                  "note": "rank-0 CUDA-event time per step over groups of `group` steps, same loop as value"}
@@ -718,11 +770,10 @@ def run_ours(args, cfg):
         note("config 4 parity: %s (%.1fs)" % (par4["ok"], par4["seconds"]))
         if not par4["ok"]:
             fail_parity(par4, "cfg4")
-        K4 = max(5, min(K, 20))
-        p4, ms4 = w4.time_value(K4, 3)
+        p4, ms4 = w4.time_value(K, 3)
         if rank == 0:
             line["cfg4"] = {"workload": "cfg4: A-softmax head fwd+bwd, C=1000000 D=512 batch=1024 m=4 lambda=5.0 bf16",
-                            "value": cfg4["B"] / (ms4[p4] * 1e-3), "unit": UNIT, "ms_per_step": ms4[p4], "steps": K4,
+                            "value": cfg4["B"] / (ms4[p4] * 1e-3), "unit": UNIT, "ms_per_step": ms4[p4], "steps": K,
                             "value_path": p4, "ms_per_step_by_path": ms4, "n_gpus": world, "scaling": "strong",
                             "parity": par4,
                             "step_algorithmic_tflops": 6.0 * cfg4["B"] * cfg4["D"] * cfg4["C"] / (ms4[p4] * 1e-3) / 1e12}
@@ -857,7 +908,12 @@ def main():
     ap.add_argument("--graph", action="store_true", help="(default) also time the CUDA-graph replay of the step")
     ap.add_argument("--no-nvlink", action="store_true", help="N>1: skip the NVLink peer-memory transport")
     ap.add_argument("--no-cfg4", action="store_true", help="skip the config-4 (C = 1M) sub-record of the cfg3 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, dX and dW (at most %d MB of dW class columns, a seeded choice) of the "
+                         "headline path's last timed step as DIR/<name>.npy, float32" % (DUMP_DW_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     cfg = dict(CONFIGS[args.workload])
     if args.mode is None:
         args.mode = cfg["mode"]

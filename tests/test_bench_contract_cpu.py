@@ -36,6 +36,63 @@ def test_reference_arm_json_line():
     assert "workload" in line["config"] and "model" not in line["config"]
 
 
+def _bench_module():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    argv, sys.argv = sys.argv, ["bench.py"]
+    try:
+        spec.loader.exec_module(b)
+    finally:
+        sys.argv = argv
+    return b
+
+
+def test_reference_arm_dumps_its_last_step(tmp_path):
+    """--dump-outputs: the loss, dX and dW the timed path returned from its last step, float32,
+    on the seeded bench inputs (config 1 is small enough for the whole dW)."""
+    import numpy as np
+    from oracle import asoftmax_ref as ref
+    from tf_face_toolbox_b200.synthetic import CONFIGS, make_inputs
+    out = tmp_path / "dump"
+    p = run("--impl", "reference", "--workload", "cfg1", "--steps", "2", "--warmup", "0", "--dump-outputs", str(out))
+    assert p.returncode == 0, p.stderr[-2000:]
+    got = {f.stem: np.load(f) for f in out.iterdir()}
+    assert sorted(got) == ["dW", "dX", "loss"] and all(a.dtype == np.float32 for a in got.values())
+    assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+    c = CONFIGS["cfg1"]
+    inp = make_inputs(c["B"], c["D"], c["C"])
+    rows = got["dX"].shape[0]                     # the reference arm may time the first rows of the batch only
+    assert got["dW"].shape == (c["D"], c["C"]) and got["dX"].shape == (rows, c["D"]) and 64 <= rows <= c["B"]
+    r = ref.asoftmax_head(inp.X[:rows].numpy(), inp.W.numpy(), inp.y[:rows].numpy(), 4, 5.0)
+    assert abs(float(got["loss"][0]) - r.loss) <= 1e-5 * r.loss
+    np.testing.assert_allclose(got["dX"], r.dX, rtol=0, atol=1e-5 * np.abs(r.dX).max())
+    np.testing.assert_allclose(got["dW"], r.dW, rtol=0, atol=1e-5 * np.abs(r.dW).max())
+
+
+def test_dumped_dw_is_a_fixed_choice_of_class_columns():
+    import numpy as np
+    import torch
+    b = _bench_module()
+    D, Cn = 512, 20000
+    dW = torch.randn(D, Cn, generator=torch.Generator().manual_seed(0))
+    res = ((torch.tensor(1.5), torch.tensor(0.25)), torch.ones(8, D), dW)
+    a, a2 = b.step_arrays(res), b.step_arrays(res)
+    assert sorted(a) == ["center_loss", "dW", "dX", "loss"]
+    assert a["loss"].tolist() == [1.5] and a["center_loss"].tolist() == [0.25]
+    keep = b.DUMP_DW_BYTES // (4 * D)
+    assert a["dW"].shape == (D, keep) and a["dW"].nbytes <= b.DUMP_DW_BYTES
+    np.testing.assert_array_equal(a["dW"], a2["dW"])
+    # the columns are whole dW columns, in increasing class order
+    cols = [int(np.nonzero((dW.numpy() == a["dW"][:, [j]]).all(axis=0))[0][0]) for j in range(0, keep, 997)]
+    assert cols == sorted(cols) and len(set(cols)) == len(cols)
+
+
+def test_steps_must_be_positive():
+    p = run("--impl", "reference", "--workload", "cfg1", "--steps", "0")
+    assert p.returncode != 0 and "--steps" in p.stderr
+
+
 def test_product_arm_has_no_cpu_fallback():
     import torch
     if torch.cuda.is_available():
@@ -80,15 +137,8 @@ def test_build_line_quotes_the_traffic_capture_of_the_same_library():
     """bench.py's line builder, fed with the recorded N = 1 measurements: the dominant kernel's
     roofline carries the per-launch DRAM traffic of the ncu capture -- and drops it for any other
     library version."""
-    import importlib.util
     import types
-    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(ROOT, "bench.py"))
-    b = importlib.util.module_from_spec(spec)
-    argv, sys.argv = sys.argv, ["bench.py"]
-    try:
-        spec.loader.exec_module(b)
-    finally:
-        sys.argv = argv
+    b = _bench_module()
     line = json.loads(open(os.path.join(ROOT, "profiles", "r2_bench_n1.json")).read().strip().splitlines()[-1])
     args = types.SimpleNamespace(workload="cfg3", gpus=1, steps=100, warmup=10, mode="bf16", impl="b200")
     cfg = {"B": 512, "D": 512, "C": 85742}
