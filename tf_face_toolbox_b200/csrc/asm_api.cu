@@ -25,7 +25,8 @@ struct asm_head {
   Step st{};                     // pointers into ws + per-step state
   size_t dx_part_capacity = 0;   // floats
   UmmaMaps maps{};
-  int maps_B = -1;
+  int maps_B = -1;               // (B, KS) the maps were encoded for: dx_st's extent is {D, B, KS}
+  int maps_KS = -1;
   bool opt_stream = false;       // ASM_OPT_STREAM=1: dW kernel + streaming update instead of the fused epilogue (opt-in)
   float* dw_scratch = nullptr;   // [D, C_local] fp32, allocated on first use of opt_stream
   bool defer_loss = true;        // ASM_DEFER_LOSS=0: combine reduces the loss itself (A/B knob)
@@ -254,10 +255,13 @@ int run_forward(asm_head* h, const float* X, int B, const void* labels, int labe
     }
     s.KS = umma_dx_splits(B, s.D, s.Cp, dx_sms(h), (h->tune.cg_mask & 8) ? 2 : 1);
     while (s.KS > 1 && (size_t)s.KS * B * s.D > h->dx_part_capacity) --s.KS;
-    if (h->maps_B != B) {
+    // KS changes at a fixed B when profiling toggles the dW / dX split (dx_sms): a stale dx_st
+    // extent would drop the stores of the splits past the old KS without an error
+    if (h->maps_B != B || h->maps_KS != s.KS) {
       if (!umma_build_maps(&h->maps, s))
         return fail(h, ASM_ERR_CUDA, "cuTensorMapEncodeTiled failed%s", "");
       h->maps_B = B;
+      h->maps_KS = s.KS;
     }
   } else {
     s.NT = simt_forward_tiles(s.C);
@@ -412,7 +416,7 @@ int asm_create(asm_head** out, const asm_config* cfg) {
   if ((e = getenv("ASM_DW_TMA"))) h->tune.dw_tma = atoi(e) != 0;
   if ((e = getenv("ASM_L2_HINTS"))) h->tune.l2_hints = (uint32_t)atoi(e);
   if ((e = getenv("ASM_UMMA_CG"))) h->tune.cg_mask = (uint32_t)atoi(e);
-  if ((e = getenv("ASM_UMMA_BN"))) h->tune.bn = (uint32_t)atoi(e);   // 128: narrow tiles (not validated on hardware yet)
+  if ((e = getenv("ASM_UMMA_BN"))) h->tune.bn = (uint32_t)atoi(e);   // 128 / 256: force the tile width
   if ((e = getenv("ASM_NO_OVERLAP")) && atoi(e)) h->overlap = false;
   // default: 57 % of the CTA pairs to the (HBM-bound) dW kernel, the rest to the (tensor-bound) dX
   // kernel -- measured at config 3: 252.8 us per step one after the other, 235.5 us side by side

@@ -10,6 +10,7 @@ from __future__ import annotations
 
 import math
 from dataclasses import dataclass
+from typing import Optional
 
 import torch
 
@@ -34,12 +35,17 @@ class HeadInputs:
     y: torch.Tensor        # [B] int32
 
 
-def make_inputs(B: int, D: int, C: int, seed: int = 1234, w_std: float = 0.01) -> HeadInputs:
+def make_inputs(B: int, D: int, C: int, seed: int = 1234, w_std: float = 0.01,
+                labels: Optional[torch.Tensor] = None) -> HeadInputs:
+    """`labels` [B] replaces the uniform draw (X is built around the given classes)."""
     gw = torch.Generator().manual_seed(seed)
     gy = torch.Generator().manual_seed(seed + 1)
     gx = torch.Generator().manual_seed(seed + 2)
     W = torch.randn(D, C, generator=gw, dtype=torch.float32) * w_std
-    y = torch.randint(0, C, (B,), generator=gy, dtype=torch.int64).to(torch.int32)
+    if labels is None:
+        y = torch.randint(0, C, (B,), generator=gy, dtype=torch.int64).to(torch.int32)
+    else:
+        y = labels.to(torch.int32).contiguous()
     wy = W[:, y.long()].t().contiguous()                        # [B, D]
     wy = wy / wy.norm(dim=1, keepdim=True)
     a = torch.tensor(MIX, dtype=torch.float32)[torch.arange(B) % 4]
