@@ -6,6 +6,7 @@ B200 A-softmax head, driven like the reference's train loop (train.py:223-250).
     python examples/train_sphereface20.py --steps 20 --batch 512 --classes 10572
     python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 \
         examples/train_sphereface20.py --batch 512        # DDP backbone + class-sharded head
+    python examples/train_sphereface20.py --margin arcface --scale 64 --margin-value 0.5
 
 Only the head is this repository's product; the backbone is ordinary PyTorch (the survey
 marks backbones out of scope) and exists to show where the head plugs in:
@@ -23,7 +24,7 @@ import torch
 import torch.nn as nn
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from tf_face_toolbox_b200 import FusedOptimizer, LambdaState, asoftmax_head  # noqa: E402
+from tf_face_toolbox_b200 import AdditiveMargin, FusedOptimizer, LambdaState, asoftmax_head  # noqa: E402
 
 
 class ResBlock(nn.Module):
@@ -87,7 +88,18 @@ def main():
     ap.add_argument("--lr", type=float, default=0.01)
     ap.add_argument("--mode", default="bf16")
     ap.add_argument("--transport", default="nvlink", help="multi-GPU exchanges: nvlink | nccl")
+    ap.add_argument("--margin", default="asoftmax", choices=["asoftmax", "arcface", "cosface"],
+                    help="A-softmax (m = 4, annealed lambda), or an additive margin on normalised embeddings")
+    ap.add_argument("--scale", type=float, default=64.0, help="s of the additive margins")
+    ap.add_argument("--margin-value", type=float, default=None,
+                    help="m2 of ArcFace (default 0.5) or m3 of CosFace (default 0.35)")
     args = ap.parse_args()
+    if args.margin == "arcface":
+        margin = AdditiveMargin.arcface(args.scale, 0.5 if args.margin_value is None else args.margin_value)
+    elif args.margin == "cosface":
+        margin = AdditiveMargin.cosface(args.scale, 0.35 if args.margin_value is None else args.margin_value)
+    else:
+        margin = None
     # under torchrun: data-parallel backbone (DDP) + class-parallel head, one rank per GPU
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -108,7 +120,8 @@ def main():
     if world > 1:
         from tf_face_toolbox_b200 import ShardedASoftmaxHead
         head = ShardedASoftmaxHead(512, args.classes, m=4, mode=args.mode, device=dev, lambda_state=lam,
-                                   transport=args.transport, batch_global=args.batch)   # N(0, 0.001) shards
+                                   transport=args.transport, batch_global=args.batch,   # N(0, 0.001) shards
+                                   margin=margin)
 
         def head_call(feats, labels):
             loss, dX, _ = head.step(feats, labels, optimizer=opt_head)                  # lambda from the clock
@@ -118,7 +131,7 @@ def main():
 
         def head_call(feats, labels):
             loss, _, dX, _ = asoftmax_head(feats, labels, args.classes, 4, lam.step(),
-                                           weights=W, mode=args.mode, optimizer=opt_head)
+                                           weights=W, mode=args.mode, optimizer=opt_head, margin=margin)
             return loss, dX
     # a fixed synthetic "dataset" of 4 batches so the loss can actually go down; every rank draws
     # the same global batch and keeps its slice (data_parallel.py:206-207)
@@ -138,7 +151,8 @@ def main():
         loss = head_step(net, images, labels, head_call, opt_backbone, world=world)
         losses.append(loss)
         if rank == 0 and (step % 5 == 0 or step == args.steps - 1):
-            print(f"step {step:4d}  cross_entropy {float(loss):.4f}  lambda {lam.value():.2f}", flush=True)
+            extra = f"  lambda {lam.value():.2f}" if margin is None else f"  {args.margin} s={margin.s:g}"
+            print(f"step {step:4d}  cross_entropy {float(loss):.4f}{extra}", flush=True)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     first, last = float(torch.stack(losses[:4]).mean()), float(torch.stack(losses[-4:]).mean())

@@ -225,6 +225,28 @@ int asm_set_gradient_transform(asm_head* h, float grad_scale, float weight_decay
  */
 int asm_set_embedding_dtype(asm_head* h, int32_t bytes_per_element);
 
+/*
+ * Margin of the target logit, per handle; it applies to every step call (asm_forward_backward,
+ * asm_forward, asm_forward_partial / asm_backward_partial, asm_step_p2p) and, like the other
+ * per-handle settings, is captured with them into a CUDA graph.
+ *   ASM_MARGIN_ASOFTMAX (default)  SphereFace: f_y = (lambda s_y + n psi(t)) / (1 + lambda) on the
+ *                                  raw embeddings, margin cfg.m.
+ *   ASM_MARGIN_ADDITIVE            L2-normalised embeddings, fixed scale s:  s_ij = s x_i.w_j / (n_i c_j),
+ *                                  t = s_iy / s,  f_y = s phi(t),  every other logit s_ij, where
+ *                                  phi(t) = cos(theta + m2) - m3        if t >= cos(pi - m2)
+ *                                         = t - m2 sin(m2) - m3          otherwise (no "easy margin").
+ *                                  m2 = 0: CosFace (s (cos theta - m3)); m3 = 0: ArcFace
+ *                                  (s cos(theta + m2)).  lambda and cfg.m are ignored.
+ * margin == NULL restores the default.  s must be finite and > 0, m2 in [0, pi/2], m3 finite and
+ * >= 0; anything else returns ASM_ERR_INVALID_ARG and changes nothing.
+ */
+enum { ASM_MARGIN_ASOFTMAX = 0, ASM_MARGIN_ADDITIVE = 1 };
+typedef struct {
+  int32_t kind;
+  float   s, m2, m3;
+} asm_margin;
+int asm_set_margin(asm_head* h, const asm_margin* margin);
+
 /* CUDA-graph support.  Kernel arguments are frozen when a step is captured into a graph, so
  * lambda (which anneals per step) can instead be read from a caller-owned DEVICE float:
  * once set (non-NULL) it overrides the by-value `lambda` argument of every step call; NULL

@@ -45,6 +45,13 @@ class AsmOptimizer(C.Structure):
 OPT_NONE, OPT_MOMENTUM, OPT_ADAM = 0, 1, 2
 
 
+class AsmMargin(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("s", C.c_float), ("m2", C.c_float), ("m3", C.c_float)]
+
+
+MARGIN_ASOFTMAX, MARGIN_ADDITIVE = 0, 1
+
+
 class AsmError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"asoftmax_b200 error {code}: {msg}")
@@ -76,6 +83,7 @@ SYMBOLS = {
     "asm_p2p_status": (C.c_int, [_P, _P]),
     "asm_set_gradient_transform": (C.c_int, [_P, C.c_float, C.c_float, _P]),
     "asm_set_embedding_dtype": (C.c_int, [_P, C.c_int32]),
+    "asm_set_margin": (C.c_int, [_P, C.POINTER(AsmMargin)]),
     "asm_set_lambda_device": (C.c_int, [_P, _P]),
     "asm_set_profiling": (C.c_int, [_P, C.c_int]),
     "asm_get_profile": (C.c_int, [_P, C.c_int32, _P, _P]),

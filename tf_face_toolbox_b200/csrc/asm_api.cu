@@ -66,8 +66,8 @@ thread_local char g_create_err[512] = "";
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct Layout {
-  size_t ylocal, flags, n, inv_n, inv_c, tgt_s, tgt_f, part, stats_local, lse, negoff, gtarget, rcoef, rowloss, counter,
-      q_part, G, dx_part, Xb, Wb, Xg, step_dev, wsq_part, wsq_ticket, total;
+  size_t ylocal, flags, n, inv_n, inv_c, margin, tgt_s, tgt_f, part, stats_local, lse, negoff, gtarget, rcoef, rowloss, counter,
+      q_part, G, dx_part, Xb, Wb, Xs, Xg, step_dev, wsq_part, wsq_ticket, total;
   int Cp, NT, MT;
   size_t dx_capacity;
 };
@@ -120,6 +120,7 @@ Layout make_layout(const asm_config& c, int num_sms) {
   L.n = take(B * 4);
   L.inv_n = take(B * 4);
   L.inv_c = take((size_t)L.Cp * 4);
+  L.margin = take(kMarginRecordFloats * 4);   // must directly precede tgt_s (margin_record)
   L.tgt_s = take(B * 4);
   L.tgt_f = take(B * 4);
   L.part = take(B * (size_t)L.NT * 8);
@@ -138,6 +139,8 @@ Layout make_layout(const asm_config& c, int num_sms) {
   if (tc) {
     L.Xb = take(planes * B * D * 2);
     L.Wb = take(planes * D * (size_t)L.Cp * 2);
+  } else {
+    L.Xs = take(B * D * 4);   // the CUDA-core kernels' scaled, normalised copy of X (additive margin)
   }
   if (c.world > 1) {
     L.Xg = take(B * D * 4);
@@ -190,6 +193,14 @@ bool split_active(const asm_head* h) {
 }
 int dw_sms(const asm_head* h) { return split_active(h) ? 2 * h->dw_pairs : h->num_sms; }
 int dx_sms(const asm_head* h) { return split_active(h) ? h->num_sms - 2 * h->dw_pairs : h->num_sms; }
+
+// The CUDA-core kernels read their embedding operand from s.X in place: with the additive margin
+// that operand is the scaled, normalised copy Xs the norm kernel wrote.
+Step simt_step(const Step& s) {
+  Step t = s;
+  if (s.mg.kind != 0) t.X = s.Xs;
+  return t;
+}
 
 // forward half up to stats_local; shared by every entry point
 int run_forward(asm_head* h, const float* X, int B, const void* labels, int label_bytes,
@@ -272,7 +283,7 @@ int run_forward(asm_head* h, const float* X, int B, const void* labels, int labe
   launch_prep(s, labels, label_bytes, stream, tp);
   mark(h, "fwd_logits_stats", stream);
   if (h->tc) launch_umma_forward(s, h->maps, h->tune, h->num_sms, stream);
-  else launch_simt_forward(s, stream);
+  else launch_simt_forward(simt_step(s), stream);
   if (want_local_stats) {
     mark(h, "combine_local", stream);
     launch_combine_local(s, stream);
@@ -309,7 +320,7 @@ int run_backward(asm_head* h, const float* stats_all, int n_shards, float* loss_
     h->tune.side_by_side = split_active(h) ? 1 : 0;
     mark(h, "bwd_recompute_g", stream);
     if (tc) launch_umma_bwdg(s, h->maps, h->tune, h->num_sms, stream);
-    else launch_simt_bwdg(s, stream);
+    else launch_simt_bwdg(simt_step(s), stream);
     // The CUDA-core dX kernel reads the fp32 master weights, which a fused optimizer rewrites in
     // the dW kernel: in that combination dX runs first, on the same stream (the tcgen05 kernels
     // read the bf16 copy, which the update never touches, so they may overlap).
@@ -325,8 +336,10 @@ int run_backward(asm_head* h, const float* stats_all, int n_shards, float* loss_
     auto run_dx = [&]() {
       mark(h, "dx_gemm", sx, !h->phase_profiling);
       if (tc) launch_umma_dx(s, h->maps, h->tune, dx_sms(h), sx);
-      else launch_simt_dx(s, sx);
-      mark(h, tp ? "dx_finish_exchange" : "dx_finish", sx, !h->phase_profiling);
+      else launch_simt_dx(simt_step(s), sx);
+      const bool add = s.mg.kind != 0;
+      mark(h, tp ? (add ? "dx_finish_margin_exchange" : "dx_finish_exchange") : (add ? "dx_finish_margin" : "dx_finish"), sx,
+           !h->phase_profiling);
       if (tp) launch_dx_finish_p2p(s, *tp, sx);
       else launch_dx_finish(s, sx);
     };
@@ -350,7 +363,7 @@ int run_backward(asm_head* h, const float* stats_all, int n_shards, float* loss_
     } else if (tc) {
       if (s.opt.kind == 0 && !s.x3 && h->tune.dw_tma) umma_build_dw_maps(&h->maps, s);
       launch_umma_dw(s, h->maps, h->tune, dw_sms(h), stream);
-    } else launch_simt_dw(s, stream);
+    } else launch_simt_dw(simt_step(s), stream);
     if (!dx_first) run_dx();
     if (fork) {
       cudaEventRecord(h->ev_join, h->side);
@@ -490,7 +503,10 @@ int asm_create(asm_head** out, const asm_config* cfg) {
   if (h->tc) {
     s.Xb = (__nv_bfloat16*)(w + L.Xb);
     s.Wb = (__nv_bfloat16*)(w + L.Wb);
+  } else {
+    s.Xs = (float*)(w + L.Xs);
   }
+  s.mg.kind = 0;
   if (cfg->world > 1) {
     h->Xg = (float*)(w + L.Xg);
     h->p2p.step_dev = (unsigned*)(w + L.step_dev);     // zeroed with the workspace
@@ -714,6 +730,28 @@ int asm_set_embedding_dtype(asm_head* h, int32_t bytes_per_element) {
   if (bytes_per_element == 2 && h->cfg.mode != ASM_MODE_BF16)
     return fail(h, ASM_ERR_INVALID_ARG, "bf16 embeddings need ASM_MODE_BF16%s", "");
   h->st.x_bf16 = bytes_per_element == 2 ? 1 : 0;
+  return ASM_OK;
+}
+
+int asm_set_margin(asm_head* h, const asm_margin* margin) {
+  if (!h) return ASM_ERR_INVALID_ARG;
+  Margin g{};
+  if (margin && margin->kind == ASM_MARGIN_ADDITIVE) {
+    const float s = margin->s, m2 = margin->m2, m3 = margin->m3;
+    if (!(isfinite(s) && s > 0.f) || !(m2 >= 0.f && m2 <= (float)(M_PI / 2)) || !(isfinite(m3) && m3 >= 0.f))
+      return fail(h, ASM_ERR_INVALID_ARG, "additive margin needs finite s > 0, m2 in [0, pi/2], finite m3 >= 0%s", "");
+    g.kind = 1;
+    g.s = s;
+    g.inv_s = (float)(1.0 / (double)s);
+    g.cm = (float)cos((double)m2);
+    g.sm = (float)sin((double)m2);
+    g.tau = (float)cos(M_PI - (double)m2);
+    g.fb = (float)((double)m2 * sin((double)m2) + (double)m3);
+    g.m3 = m3;
+  } else if (margin && margin->kind != ASM_MARGIN_ASOFTMAX) {
+    return fail(h, ASM_ERR_INVALID_ARG, "unknown margin kind%s", "");
+  }
+  h->st.mg = g;
   return ASM_OK;
 }
 

@@ -40,6 +40,50 @@ __device__ __forceinline__ void psi_eval(float t, int m, float& psi, float& dpsi
   dpsi = sgn * dT;
 }
 
+// ---------------------------------------------------------------------------------------
+// Additive margin on L2-normalised embeddings (asm_set_margin, DESIGN.md section 2.1).  The
+// GEMMs then see s * x_i / n_i, so a raw logit is s * cos(theta) and t = logit / s.
+//   t >= tau = cos(pi - m2):  phi = cos(theta + m2) - m3,  phi' = cos m2 + t sin m2 / sin(theta)
+//   otherwise:                phi = t - m2 sin m2 - m3,    phi' = 1
+// (the usual non-"easy-margin" fallback; phi jumps at tau).  kind == 0: A-softmax instead.
+// ---------------------------------------------------------------------------------------
+struct Margin {
+  int kind;                  // 0 = A-softmax (psi, lambda), 1 = additive (s, m2, m3)
+  float s, inv_s;            // scale and 1/s
+  float cm, sm;              // cos m2, sin m2
+  float tau;                 // cos(pi - m2)
+  float fb;                  // m2 sin m2 + m3: offset of the fallback branch
+  float m3;
+};
+
+__device__ __forceinline__ void phi_eval(float t, const Margin& g, float& phi, float& dphi) {
+  t = fminf(1.0f, fmaxf(-1.0f, t));
+  if (t >= g.tau) {
+    const float st = sqrtf(fmaxf(1.0f - t * t, 1e-12f));
+    phi = t * g.cm - st * g.sm - g.m3;
+    dphi = g.cm + t * g.sm / st;
+  } else {
+    phi = t - g.fb;
+    dphi = 1.0f;
+  }
+}
+
+// The norm kernel copies the step's Margin into the workspace slot of kMarginRecordFloats floats
+// that directly precedes tgt_s (asm_api.cu, make_layout), where the forward GEMM's out-of-line
+// target patch finds it without an argument of its own.
+constexpr int kMarginRecordFloats = 64;
+static_assert(sizeof(Margin) <= kMarginRecordFloats * sizeof(float), "margin record slot");
+__device__ __forceinline__ const Margin* margin_record(const float* tgt_s) {
+  return reinterpret_cast<const Margin*>(tgt_s - kMarginRecordFloats);
+}
+
+// f_{i,y} = s * phi(s_y / s)
+__device__ __forceinline__ float additive_logit(float sv, const Margin& g) {
+  float phi, dphi;
+  phi_eval(sv * g.inv_s, g, phi, dphi);
+  return g.s * phi;
+}
+
 // f_{i,y} = (lambda * s + n * psi(s/n)) / (1 + lambda)
 __device__ __forceinline__ float target_logit(float s, float n, float inv_n, int m, float lambda) {
   float psi, dpsi;

@@ -5,6 +5,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "asm_common.cuh"
+
 namespace asmh {
 
 // Everything one step needs; filled by the host API (asm_api.cu), passed by value.
@@ -161,6 +163,11 @@ struct Step {
   int l2_hints;              // evict-first on single-use streams (the fp32 W read of the norm kernel)
   int pdl;                   // launch dependents programmatically (eager, non-captured streams)
   int defer_loss;            // the mean-loss reduction runs in an idle warp of the dX kernel, not in combine
+  // margin of the target logit (asm_set_margin).  Additive kind: the norm kernel writes the operand
+  // copies of s * x_i / n_i (n, inv_n and X stay the true embeddings, for dx_finish), the forward
+  // patches s * phi(t) in, combine sets G'_y = g_y phi'(t) and r = 0, dx_finish projects each row.
+  Margin mg;
+  float* Xs;                 // [B, D] fp32 s * x_i / n_i: what the CUDA-core kernels read in place of X (additive kind)
 };
 
 // prep: column norms of W (+ bf16 copy), row norms of X (+ bf16 copy), label localisation.
@@ -177,7 +184,7 @@ void launch_combine_local(const Step& s, cudaStream_t st);
 void launch_combine_global(const Step& s, const float* stats_all, int n_shards, cudaStream_t st);
 // single shard: both of the above in one launch (partials -> stats_local, lse, loss, ...)
 void launch_combine_fused(const Step& s, cudaStream_t st);
-// dX = sum_z dx_part[z] + r_i x_i
+// dX = sum_z dx_part[z] + r_i x_i; additive kind: dX_i = (s/n_i)(v_i - (x_i.v_i)/n_i^2 x_i), v_i = sum_z dx_part[z]
 void launch_dx_finish(const Step& s, cudaStream_t st);
 // streaming classifier update from a dW buffer (alternative to the fused dW epilogue)
 void launch_opt_stream(const Step& s, const float* dW, cudaStream_t st);

@@ -117,12 +117,7 @@ void launch_combine_p2p(const Step& s, const P2P& p, cudaStream_t st) {
 // kernel of the step, this one included, has read it by then).  Only the last kReducers blocks
 // stay for the exchange (p.waiters: so at most that many blocks ever spin on a peer), wait for every
 // rank's flag and sum this rank's rows over the shards in rank order (deterministic).
-template <int KS_T>
-__global__ void __launch_bounds__(256) dx_finish_p2p_kernel(Step s, P2P p) {
-  pdl_trigger();
-  pdl_wait();
-  const unsigned cur = p2p_current_step(p);
-  dx_finish_rows<KS_T>(s, p.dx(p.rank, cur & 1), blockIdx.x, gridDim.x);
+__device__ __forceinline__ void dx_exchange(const Step& s, const P2P& p, unsigned cur) {
   const unsigned n = gridDim.x;
   const unsigned tk = block_ticket(p.tickets + 2, n);
   if (tk == n - 1 && threadIdx.x == 0) {
@@ -154,7 +149,33 @@ __global__ void __launch_bounds__(256) dx_finish_p2p_kernel(Step s, P2P p) {
   }
 }
 
+template <int KS_T>
+__global__ void __launch_bounds__(256) dx_finish_p2p_kernel(Step s, P2P p) {
+  pdl_trigger();
+  pdl_wait();
+  const unsigned cur = p2p_current_step(p);
+  dx_finish_rows<KS_T>(s, p.dx(p.rank, cur & 1), blockIdx.x, gridDim.x);
+  dx_exchange(s, p, cur);
+}
+
+// additive margin: this shard projects its own partial sum of every row before it publishes it
+// (the projection is linear in v); the rank-order sum of the exchange is unchanged
+__global__ void __launch_bounds__(256) dx_finish_margin_p2p_kernel(Step s, P2P p) {
+  __shared__ float red[8];
+  pdl_trigger();
+  pdl_wait();
+  const unsigned cur = p2p_current_step(p);
+  dx_finish_rows_margin(s, p.dx(p.rank, cur & 1), blockIdx.x, gridDim.x, red);
+  dx_exchange(s, p, cur);
+}
+
 void launch_dx_finish_p2p(const Step& s, const P2P& p, cudaStream_t st) {
+  if (s.mg.kind != 0) {
+    int blocks = (s.B + 1) / 2;
+    if (blocks > 148 * 2) blocks = 148 * 2;
+    launch_pdl(dx_finish_margin_p2p_kernel, dim3(blocks), dim3(256), 0, st, s.pdl != 0, 1, s, p);
+    return;
+  }
   const size_t total4 = (size_t)s.B * s.D / 4;
   int blocks = (int)((total4 + 255) / 256);
   if (blocks > 148 * 2) blocks = 148 * 2;
@@ -176,6 +197,7 @@ void p2p_preload_kernels() {
   cudaFuncGetAttributes(&a, dx_finish_p2p_kernel<9>);
   cudaFuncGetAttributes(&a, dx_finish_p2p_kernel<4>);
   cudaFuncGetAttributes(&a, dx_finish_p2p_kernel<0>);
+  cudaFuncGetAttributes(&a, dx_finish_margin_p2p_kernel);
   prep_preload_kernels();
   simt_preload_kernels();
   cudaGetLastError();

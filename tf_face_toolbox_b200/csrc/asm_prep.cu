@@ -25,8 +25,108 @@ namespace asmh {
 // the W role, which depends on nobody, runs meanwhile.  Publish blocks come first in the grid
 // so that they are dispatched before any block that waits for a peer.
 // ---------------------------------------------------------------------------------------
-// vblock: the block index this call plays (blockIdx.x)
-template <bool VEC2, int PL, int TX, int TY, int U>
+// Per-row results of the X role (lane 0 of the row's warp): norm, 1/norm, local label.
+__device__ __forceinline__ void prep_row_tail(const Step& s, int row, float acc, long long y) {
+  const float nn = sqrtf(acc);
+  s.n[row] = nn;
+  s.inv_n[row] = nn > 0.f ? 1.0f / nn : 0.f;
+  // -1: owned by another shard; -2: outside [0, C_total) (reported by asm_check_labels, and
+  // the row's loss becomes NaN; both mean "no target column here" to the GEMM kernels, so a
+  // bad label never faults)
+  const long long yl = y - s.class_offset;
+  s.ylocal[row] = (y < 0 || y >= s.C_total) ? -2 : ((yl >= 0 && yl < s.C) ? (int)yl : -1);
+  s.tgt_s[row] = 0.f;
+  s.tgt_f[row] = 0.f;
+}
+
+// X role for the additive margin (one warp per row): the operand copies hold fl(x * (s/n)), so
+// n must be known before the first plane is written.  Pass 1 reads the row (and, on the NVLink
+// path, stores the gathered copy Xg) and reduces |x|^2; pass 2 writes the PL bf16 planes of the
+// scaled row, or with PL == 0 (CUDA-core fp32 path) the fp32 copy Xs.  A row of up to 128
+// 16-byte pieces (D <= 512 fp32, D <= 1024 bf16) stays in registers; a longer one is read again
+// (from Xg on the NVLink path: this lane wrote those pieces itself).  n / inv_n stay the true norm.
+template <int PL>
+__device__ __forceinline__ void prep_row_scaled(const Step& s, const char* x, char* xg, int esz, bool gather,
+                                                int row, long long y) {
+  const int tx = threadIdx.x & 31;
+  const float4* x4 = reinterpret_cast<const float4*>(x);
+  const int n16 = s.D * esz / 16;
+  const int epp = 16 / esz;
+  auto sq16 = [&](const float4& v) {
+    if (esz == 2) {
+      const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&v);
+      float a = 0.f;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const float l = __low2float(h2[q]), h = __high2float(h2[q]);
+        a = fmaf(l, l, a);
+        a = fmaf(h, h, a);
+      }
+      return a;
+    }
+    return fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, v.w * v.w)));
+  };
+  float4 v[4];
+  float acc = 0.f;
+  for (int i0 = 0; i0 < n16; i0 += 128) {
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + u * 32 + tx;
+      v[u] = i < n16 ? (gather ? __ldcv(x4 + i) : __ldg(x4 + i)) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + u * 32 + tx;
+      if (i < n16) {
+        if (gather) reinterpret_cast<float4*>(xg)[i] = v[u];
+        acc += sq16(v[u]);
+      }
+    }
+  }
+  acc = warp_sum(acc);
+  const float nn = sqrtf(acc);
+  const float sc = nn > 0.f ? s.mg.s / nn : 0.f;
+  auto put = [&](int d, float e) {
+    const float u = e * sc;
+    if (PL > 0) {
+      __nv_bfloat16* dst = s.Xb + (size_t)row * PL * s.D + d;
+      float r = u;
+#pragma unroll
+      for (int p2 = 0; p2 < PL; ++p2) {
+        const __nv_bfloat16 hv = __float2bfloat16_rn(r);
+        dst[(size_t)p2 * s.D] = hv;
+        r -= __bfloat162float(hv);
+      }
+    } else {
+      s.Xs[(size_t)row * s.D + d] = u;
+    }
+  };
+  auto put16 = [&](int e0, const float4& w) {
+    if (esz == 2) {
+      const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&w);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        put(e0 + 2 * q, __low2float(h2[q]));
+        put(e0 + 2 * q + 1, __high2float(h2[q]));
+      }
+    } else {
+      put(e0, w.x); put(e0 + 1, w.y); put(e0 + 2, w.z); put(e0 + 3, w.w);
+    }
+  };
+  const float4* again = gather ? reinterpret_cast<const float4*>(xg) : x4;
+  for (int i0 = 0; i0 < n16; i0 += 128) {
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + u * 32 + tx;
+      if (i < n16) put16(i * epp, n16 <= 128 ? v[u] : again[i]);
+    }
+  }
+  if (tx == 0) prep_row_tail(s, row, acc, y);
+}
+
+// vblock: the block index this call plays (blockIdx.x).  ADD: the additive-margin X role
+// (prep_row_scaled), a separate instantiation so that it costs the A-softmax kernels no registers.
+template <bool VEC2, int PL, int TX, int TY, int U, bool ADD>
 __device__ __forceinline__ void prep_block(const Step& s, const void* labels, int label_bytes,
                                            int nwb, int npub, const P2P& p, const int vblock,
                                            float (*red)[2 * TX]) {
@@ -158,6 +258,10 @@ __device__ __forceinline__ void prep_block(const Step& s, const void* labels, in
       y = label_bytes == 8 ? reinterpret_cast<const long long*>(labels)[row]
                            : (long long)reinterpret_cast<const int*>(labels)[row];
     }
+    if (ADD) {
+      prep_row_scaled<PL>(s, x, xg, esz, npub > 0, row, y);
+      return;
+    }
     float acc = 0.f;
     auto emit = [&](int d, float v) {               // one element: norm, bf16 planes
       acc = fmaf(v, v, acc);
@@ -208,30 +312,20 @@ __device__ __forceinline__ void prep_block(const Step& s, const void* labels, in
       }
     }
     acc = warp_sum(acc);
-    if (tx == 0) {
-      const float nn = sqrtf(acc);
-      s.n[row] = nn;
-      s.inv_n[row] = nn > 0.f ? 1.0f / nn : 0.f;
-      // -1: owned by another shard; -2: outside [0, C_total) (reported by asm_check_labels, and
-      // the row's loss becomes NaN; both mean "no target column here" to the GEMM kernels, so a
-      // bad label never faults)
-      const long long yl = y - s.class_offset;
-      s.ylocal[row] = (y < 0 || y >= s.C_total) ? -2 : ((yl >= 0 && yl < s.C) ? (int)yl : -1);
-      s.tgt_s[row] = 0.f;
-      s.tgt_f[row] = 0.f;
-    }
+    if (tx == 0) prep_row_tail(s, row, acc, y);
   }
 }
 
-template <bool VEC2, int PL, int TX, int TY, int U>
+template <bool VEC2, int PL, int TX, int TY, int U, bool ADD>
 __global__ void __launch_bounds__(256) prep_kernel(Step s, const void* labels, int label_bytes,
                                                    int nwb, int npub, P2P p) {
   pdl_trigger();            // first kernel of the step: nothing to wait for
   __shared__ float red[TY][2 * TX];
-  prep_block<VEC2, PL, TX, TY, U>(s, labels, label_bytes, nwb, npub, p, (int)blockIdx.x, red);
+  if (blockIdx.x == 0 && threadIdx.x == 0) *const_cast<Margin*>(margin_record(s.tgt_s)) = s.mg;
+  prep_block<VEC2, PL, TX, TY, U, ADD>(s, labels, label_bytes, nwb, npub, p, (int)blockIdx.x, red);
 }
 
-template <int TX, int TY, int U>
+template <int TX, int TY, int U, bool ADD>
 static void launch_prep_t(const Step& s, const void* labels, int label_bytes, cudaStream_t st, const P2P* p) {
   const int nwb = (s.Cp + 2 * TX - 1) / (2 * TX);
   const int nxb = (s.B + 7) / 8;
@@ -246,15 +340,21 @@ static void launch_prep_t(const Step& s, const void* labels, int label_bytes, cu
   const bool vec2 = (s.C % 2 == 0) && ((reinterpret_cast<uintptr_t>(s.W) & 7) == 0);
   dim3 grd(npub + nwb + nxb);
   if (s.x3) {
-    if (vec2) prep_kernel<true, 3, TX, TY, U><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
-    else prep_kernel<false, 3, TX, TY, U><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
+    if (vec2) prep_kernel<true, 3, TX, TY, U, ADD><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
+    else prep_kernel<false, 3, TX, TY, U, ADD><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
   } else if (s.mode == 1) {
-    if (vec2) prep_kernel<true, 1, TX, TY, U><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
-    else prep_kernel<false, 1, TX, TY, U><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
+    if (vec2) prep_kernel<true, 1, TX, TY, U, ADD><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
+    else prep_kernel<false, 1, TX, TY, U, ADD><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
   } else {
-    if (vec2) prep_kernel<true, 0, TX, TY, U><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
-    else prep_kernel<false, 0, TX, TY, U><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
+    if (vec2) prep_kernel<true, 0, TX, TY, U, ADD><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
+    else prep_kernel<false, 0, TX, TY, U, ADD><<<grd, 256, 0, st>>>(s, labels, label_bytes, nwb, npub, pp);
   }
+}
+
+template <int TX, int TY, int U>
+static void launch_prep_t(const Step& s, const void* labels, int label_bytes, cudaStream_t st, const P2P* p) {
+  if (s.mg.kind != 0) launch_prep_t<TX, TY, U, true>(s, labels, label_bytes, st, p);
+  else launch_prep_t<TX, TY, U, false>(s, labels, label_bytes, st, p);
 }
 
 void launch_prep(const Step& s, const void* labels, int label_bytes, cudaStream_t st, const P2P* p) {
@@ -387,6 +487,7 @@ void launch_combine_fused(const Step& s, cudaStream_t st) {
 
 // ---------------------------------------------------------------------------------------
 // dx_finish: dX = sum_z dx_part[z] + r_i * x_i   (float4 along D; D % 4 == 0)
+// additive margin: dX_i = (s/n_i) (v_i - (x_i.v_i)/n_i^2 x_i),  v_i = sum_z dx_part[z][i]
 // ---------------------------------------------------------------------------------------
 template <int KS_T>
 __global__ void __launch_bounds__(256) dx_finish_kernel(Step s) {
@@ -395,7 +496,21 @@ __global__ void __launch_bounds__(256) dx_finish_kernel(Step s) {
   dx_finish_rows<KS_T>(s, s.dX, blockIdx.x, gridDim.x);
 }
 
+// additive margin: the same sum, then each row projected onto the tangent space of x_i (two rows per block)
+__global__ void __launch_bounds__(256) dx_finish_margin_kernel(Step s) {
+  __shared__ float red[8];
+  pdl_trigger();
+  pdl_wait();
+  dx_finish_rows_margin(s, s.dX, blockIdx.x, gridDim.x, red);
+}
+
 void launch_dx_finish(const Step& s, cudaStream_t st) {
+  if (s.mg.kind != 0) {
+    int blocks = (s.B + 1) / 2;
+    if (blocks > 148 * 8) blocks = 148 * 8;
+    launch_pdl(dx_finish_margin_kernel, dim3(blocks), dim3(256), 0, st, s.pdl != 0, 1, s);
+    return;
+  }
   const size_t total4 = (size_t)s.B * s.D / 4;
   int blocks = (int)((total4 + 255) / 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
@@ -462,15 +577,20 @@ void launch_opt_stream(const Step& s, const float* dW, cudaStream_t st) {
   }
 }
 
-template <int TX, int TY, int U>
+template <int TX, int TY, int U, bool ADD>
 static void preload_prep_t() {
   cudaFuncAttributes a;
-  cudaFuncGetAttributes(&a, prep_kernel<true, 3, TX, TY, U>);
-  cudaFuncGetAttributes(&a, prep_kernel<false, 3, TX, TY, U>);
-  cudaFuncGetAttributes(&a, prep_kernel<true, 1, TX, TY, U>);
-  cudaFuncGetAttributes(&a, prep_kernel<false, 1, TX, TY, U>);
-  cudaFuncGetAttributes(&a, prep_kernel<true, 0, TX, TY, U>);
-  cudaFuncGetAttributes(&a, prep_kernel<false, 0, TX, TY, U>);
+  cudaFuncGetAttributes(&a, prep_kernel<true, 3, TX, TY, U, ADD>);
+  cudaFuncGetAttributes(&a, prep_kernel<false, 3, TX, TY, U, ADD>);
+  cudaFuncGetAttributes(&a, prep_kernel<true, 1, TX, TY, U, ADD>);
+  cudaFuncGetAttributes(&a, prep_kernel<false, 1, TX, TY, U, ADD>);
+  cudaFuncGetAttributes(&a, prep_kernel<true, 0, TX, TY, U, ADD>);
+  cudaFuncGetAttributes(&a, prep_kernel<false, 0, TX, TY, U, ADD>);
+}
+template <int TX, int TY, int U>
+static void preload_prep_t() {
+  preload_prep_t<TX, TY, U, false>();
+  preload_prep_t<TX, TY, U, true>();
 }
 void prep_preload_kernels() {
   preload_prep_t<16, 16, 8>();
@@ -482,6 +602,7 @@ void prep_preload_kernels() {
   cudaFuncGetAttributes(&a, combine_kernel<true>);
   cudaFuncGetAttributes(&a, combine_kernel<false>);
   cudaFuncGetAttributes(&a, dx_finish_kernel<0>);
+  cudaFuncGetAttributes(&a, dx_finish_margin_kernel);
   cudaFuncGetAttributes(&a, opt_stream_kernel<4>);
   cudaFuncGetAttributes(&a, opt_stream_kernel<1>);
 }

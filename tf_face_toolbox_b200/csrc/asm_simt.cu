@@ -165,7 +165,8 @@ __global__ void __launch_bounds__(256) simt_kernel(Step s, int k_per_split) {
         float v = acc[a][b] * ic[b];
         if (rv && j == yl) {
           s.tgt_s[i] = v;
-          v = target_logit(v, s.n[i], s.inv_n[i], s.m, step_lambda(s.lambda, s.lambda_dev));
+          v = s.mg.kind != 0 ? additive_logit(v, s.mg)
+                             : target_logit(v, s.n[i], s.inv_n[i], s.m, step_lambda(s.lambda, s.lambda_dev));
           s.tgt_f[i] = v;
         }
         if (j >= s.C) v = -INFINITY;

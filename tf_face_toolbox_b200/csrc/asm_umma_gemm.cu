@@ -135,11 +135,14 @@ __device__ __forceinline__ float sel_eq(int i, int k, float a, float b) {
   return r;
 }
 // Rare paths of the forward epilogue, kept out of line so the hot loop stays small.
+// The margin comes from the record the norm kernel stored in front of tgt_s: an extra argument
+// would change the register allocation of the forward kernel's hot loop.
 __device__ __noinline__ float fwd_target(float* tgt_s, float* tgt_f, const float* n,
                                          const float* inv_n, int m, float lambda, int row,
                                          float sv) {
   tgt_s[row] = sv;
-  const float fv = target_logit(sv, n[row], inv_n[row], m, lambda);
+  const Margin mg = *margin_record(tgt_s);
+  const float fv = mg.kind != 0 ? additive_logit(sv, mg) : target_logit(sv, n[row], inv_n[row], m, lambda);
   tgt_f[row] = fv;
   return fv;
 }

@@ -57,6 +57,34 @@ class LambdaState:
         return self.value()
 
 
+# --------------------------------------------------------------------------------------
+# additive-margin heads (ArcFace / CosFace) on L2-normalised embeddings
+# --------------------------------------------------------------------------------------
+@dataclass(frozen=True)
+class AdditiveMargin:
+    """Target logit s * phi(cos theta) on normalised embeddings and weights, every other logit
+    s * cos(theta_j), with phi(t) = cos(theta + m2) - m3 for t >= cos(pi - m2) and
+    t - m2 sin(m2) - m3 below that (InsightFace's combined margin without m1; no "easy margin").
+    m2 = 0 is CosFace, m3 = 0 is ArcFace.  Pass it as `margin=` to the head's entry points;
+    `m` and lambda are then ignored.  s > 0, 0 <= m2 <= pi/2 and m3 >= 0 are checked by the library."""
+    s: float = 64.0
+    m2: float = 0.5
+    m3: float = 0.0
+
+    @classmethod
+    def arcface(cls, s: float = 64.0, m: float = 0.5) -> "AdditiveMargin":
+        """s * cos(theta + m)."""
+        return cls(float(s), float(m), 0.0)
+
+    @classmethod
+    def cosface(cls, s: float = 64.0, m: float = 0.35) -> "AdditiveMargin":
+        """s * (cos(theta) - m)."""
+        return cls(float(s), 0.0, float(m))
+
+    def _struct(self) -> "_lib.AsmMargin":
+        return _lib.AsmMargin(_lib.MARGIN_ADDITIVE, self.s, self.m2, self.m3)
+
+
 def _as_lambda(lambda_state) -> float:
     if lambda_state is None:
         return 0.0
@@ -66,11 +94,12 @@ def _as_lambda(lambda_state) -> float:
 
 
 # --------------------------------------------------------------------------------------
-# handle cache: one asm_head per (device, shard geometry, B_max, m, mode)
+# handle cache: one asm_head per (device, shard geometry, B_max, m, mode, margin)
 # --------------------------------------------------------------------------------------
 class _Handle:
     def __init__(self, device: torch.device, D: int, C_total: int, C_local: int, class_offset: int,
-                 B_max: int, m: int, mode: str, rank: int = 0, world: int = 1):
+                 B_max: int, m: int, mode: str, rank: int = 0, world: int = 1,
+                 margin: Optional[AdditiveMargin] = None):
         self.lib = _lib.load()
         if device.type != "cuda":
             raise RuntimeError("the A-softmax head runs on a CUDA (B200) device only; no CPU fallback")
@@ -82,6 +111,13 @@ class _Handle:
             rc = self.lib.asm_create(C.byref(self.ptr), C.byref(self.cfg))
         if rc != _lib.ASM_OK:
             raise _lib.AsmError(rc, (self.lib.asm_last_error(None) or b"").decode())
+        if margin is not None:
+            # set once: the margin is part of the handle-cache key, never switched per call
+            rc = self.lib.asm_set_margin(self.ptr, C.byref(margin._struct()))
+            if rc != _lib.ASM_OK:
+                err = _lib.AsmError(rc, (self.lib.asm_last_error(self.ptr) or b"").decode())
+                self.close()
+                raise err
 
     def close(self):
         if self.ptr:
@@ -107,16 +143,19 @@ def _round_batch(B: int) -> int:
     return max(128, (B + 127) // 128 * 128)
 
 
-def get_handle(device, D, C_total, C_local, class_offset, B, m, mode, rank=0, world=1, tag=None) -> _Handle:
+def get_handle(device, D, C_total, C_local, class_offset, B, m, mode, rank=0, world=1, tag=None,
+               margin: Optional[AdditiveMargin] = None) -> _Handle:
     """`tag` separates handles with different per-handle state (e.g. a CUDA-graph step that
     reads lambda from device memory) from the plain eager ones."""
     device = torch.device(device)
     if device.index is None:
         device = torch.device("cuda", torch.cuda.current_device())
-    key = (device.index, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, tag)
+    if margin is not None and not isinstance(margin, AdditiveMargin):
+        raise TypeError("margin must be None (A-softmax) or an AdditiveMargin")
+    key = (device.index, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin, tag)
     h = _HANDLES.get(key)
     if h is None:
-        h = _Handle(device, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world)
+        h = _Handle(device, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin)
         h.key = key
         _HANDLES[key] = h
         untagged = [k for k in _HANDLES if k[-1] is None]
@@ -200,7 +239,8 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
                   return_logits: bool = False, compute_grads: bool = True,
                   check_labels: bool = False, optimizer: Optional["FusedOptimizer"] = None,
                   grad_scale: float = 1.0, weight_decay: float = 0.0,
-                  reg_loss_out: Optional[torch.Tensor] = None, _handle_tag=None
+                  reg_loss_out: Optional[torch.Tensor] = None, margin: Optional[AdditiveMargin] = None,
+                  _handle_tag=None
                   ) -> Tuple[torch.Tensor, Optional[torch.Tensor], Optional[torch.Tensor], Optional[torch.Tensor]]:
     """A-softmax head forward + backward on one GPU that owns every class.
 
@@ -217,6 +257,8 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
     (mult_lr / num_gpus, data_parallel.py:37), dW includes weight_decay * W (the gradient of
     reg_loss, nets/sphere.py:88) and reg_loss_out (a 1-element CUDA float tensor) receives
     weight_decay/2 * |W|^2 (nets/net_base.py:103-107).  The returned loss is the plain cross-entropy.
+    `margin` (an AdditiveMargin) selects the ArcFace / CosFace head on normalised embeddings
+    instead of A-softmax; `m` and lambda_state are then ignored.  None: A-softmax.
     Asynchronous on the current CUDA stream.
     """
     _check_inputs(embeddings, labels, weights, num_classes)
@@ -229,7 +271,7 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
     y = labels.contiguous()
     B, D = X.shape
     Cn = W.shape[1]
-    h = get_handle(X.device, D, Cn, Cn, 0, B, m, mode, tag=_handle_tag)
+    h = get_handle(X.device, D, Cn, Cn, 0, B, m, mode, tag=_handle_tag, margin=margin)
     lam = _as_lambda(lambda_state)
     loss = torch.empty(1, device=X.device, dtype=torch.float32)
     logits = torch.empty(B, Cn, device=X.device, dtype=torch.float32) if return_logits else None
@@ -294,7 +336,7 @@ class GraphedASoftmaxStep:
     """
 
     def __init__(self, weights: torch.Tensor, batch_size: int, m: int = 4, mode: str = "bf16",
-                 labels_dtype=torch.int32):
+                 labels_dtype=torch.int32, margin: Optional[AdditiveMargin] = None):
         assert weights.is_cuda and weights.dtype == torch.float32 and weights.is_contiguous()
         dev = weights.device
         self.W = weights
@@ -303,9 +345,9 @@ class GraphedASoftmaxStep:
         self.y = torch.zeros(batch_size, device=dev, dtype=labels_dtype)
         self.lam = torch.zeros(1, device=dev, dtype=torch.float32)
         self._lam_host = torch.zeros(1, dtype=torch.float32).pin_memory()
-        self.m, self.mode, self.Cn = m, mode, Cn
+        self.m, self.mode, self.Cn, self.margin = m, mode, Cn, margin
         self._tag = ("graph", id(self))
-        h = get_handle(dev, D, Cn, Cn, 0, batch_size, m, mode, tag=self._tag)
+        h = get_handle(dev, D, Cn, Cn, 0, batch_size, m, mode, tag=self._tag, margin=margin)
         self._key = h.key
         _lib.check(h.lib.asm_set_lambda_device(h.ptr, self.lam.data_ptr()), h.ptr)
         cur = torch.cuda.current_stream(dev)
@@ -322,7 +364,7 @@ class GraphedASoftmaxStep:
 
     def _run(self):
         loss, _, dX, dW = asoftmax_head(self.X, self.y, self.Cn, self.m, 0.0, weights=self.W,
-                                        mode=self.mode, _handle_tag=self._tag)
+                                        mode=self.mode, margin=self.margin, _handle_tag=self._tag)
         return loss, dX, dW
 
     def close(self):
@@ -352,16 +394,17 @@ class GraphedASoftmaxStep:
 # torch autograd bridge: lets a torch backbone train through the fused head
 # --------------------------------------------------------------------------------------
 class ASoftmaxLoss(torch.autograd.Function):
-    """loss = ASoftmaxLoss.apply(embeddings, weights, labels, m, lam, mode[, upstream]).  The fused
+    """loss = ASoftmaxLoss.apply(embeddings, weights, labels, m, lam, mode[, upstream[, margin]]).  The fused
     call already produced dX and dW, so backward only hands them on.  `upstream` (a float) is the
     gradient the caller promises to send into this loss (1.0 for a plain `loss.backward()`, the loss
     scale otherwise): it is applied inside the kernels and backward returns the stored gradients
-    untouched -- no pass over [D, C].  Without it backward multiplies by the incoming gradient."""
+    untouched -- no pass over [D, C].  Without it backward multiplies by the incoming gradient.
+    `margin` (an AdditiveMargin, or None for A-softmax) as in asoftmax_head."""
 
     @staticmethod
-    def forward(ctx, embeddings, weights, labels, m, lam, mode, upstream=None):
+    def forward(ctx, embeddings, weights, labels, m, lam, mode, upstream=None, margin=None):
         loss, _, dX, dW = asoftmax_head(embeddings, labels, weights.shape[1], m, lam, weights=weights, mode=mode,
-                                        grad_scale=1.0 if upstream is None else float(upstream))
+                                        grad_scale=1.0 if upstream is None else float(upstream), margin=margin)
         ctx.save_for_backward(dX, dW)
         ctx.upstream = upstream
         return loss
@@ -370,8 +413,8 @@ class ASoftmaxLoss(torch.autograd.Function):
     def backward(ctx, grad_out):
         dX, dW = ctx.saved_tensors
         if ctx.upstream is not None:
-            return dX, dW, None, None, None, None, None
-        return grad_out * dX, grad_out * dW, None, None, None, None, None
+            return dX, dW, None, None, None, None, None, None
+        return grad_out * dX, grad_out * dW, None, None, None, None, None, None
 
 
 # --------------------------------------------------------------------------------------
@@ -392,7 +435,7 @@ class ASoftmaxHead:
     def __init__(self, num_features: int, num_classes: int, m: int = 4, weight_decay: float = 5e-4,
                  mode: str = "bf16", device="cuda", lambda_state: Optional[LambdaState] = None,
                  return_logits: bool = False, seed: Optional[int] = None, num_gpus: int = 1,
-                 mult_lr: float = 1.0):
+                 mult_lr: float = 1.0, margin: Optional[AdditiveMargin] = None):
         gen = None
         if seed is not None:
             gen = torch.Generator(device="cpu").manual_seed(seed)
@@ -401,6 +444,7 @@ class ASoftmaxHead:
         self.weights = w.to(device)                  # classifier/fc_classifier/weights [D, C]
         self.num_classes = num_classes
         self.m = m
+        self.margin = margin                         # None: A-softmax; AdditiveMargin: ArcFace / CosFace
         self.weight_decay = weight_decay
         self.mode = mode
         self.lambda_state = lambda_state if lambda_state is not None else LambdaState()
@@ -422,7 +466,8 @@ class ASoftmaxHead:
         loss, logits, dX, dW = asoftmax_head(features, labels, num_classes, self.m, lam,
                                              weights=self.weights, mode=self.mode,
                                              return_logits=self.return_logits, grad_scale=scale,
-                                             weight_decay=self.weight_decay, reg_loss_out=self._reg)
+                                             weight_decay=self.weight_decay, reg_loss_out=self._reg,
+                                             margin=self.margin)
         self._last = dict(loss=loss, dX=dX, dW=dW, lam=lam, scale=scale, reg=self._reg[0].clone())
         out = {"logits": logits, "features": features}
         return out
@@ -437,7 +482,8 @@ class ASoftmaxHead:
         losses.append(self._last["reg"])
         losses_name.append("reg_loss")
         others = OrderedDict()
-        others["lambda"] = self._last["lam"]
+        if self.margin is None:                       # lambda means nothing to the additive margins
+            others["lambda"] = self._last["lam"]
         return losses, losses_name, others
 
     def gradients(self, num_gpus: Optional[int] = None, mult_lr: Optional[float] = None):
