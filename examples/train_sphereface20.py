@@ -7,6 +7,7 @@ B200 A-softmax head, driven like the reference's train loop (train.py:223-250).
     python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 \
         examples/train_sphereface20.py --batch 512        # DDP backbone + class-sharded head
     python examples/train_sphereface20.py --margin arcface --scale 64 --margin-value 0.5
+    python examples/train_sphereface20.py --loss focal --focal-gamma 1 --focal-alpha 2
 
 Only the head is this repository's product; the backbone is ordinary PyTorch (the survey
 marks backbones out of scope) and exists to show where the head plugs in:
@@ -24,7 +25,7 @@ import torch
 import torch.nn as nn
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from tf_face_toolbox_b200 import AdditiveMargin, FusedOptimizer, LambdaState, asoftmax_head  # noqa: E402
+from tf_face_toolbox_b200 import AdditiveMargin, FocalLoss, FusedOptimizer, LambdaState, asoftmax_head  # noqa: E402
 
 
 class ResBlock(nn.Module):
@@ -93,7 +94,12 @@ def main():
     ap.add_argument("--scale", type=float, default=64.0, help="s of the additive margins")
     ap.add_argument("--margin-value", type=float, default=None,
                     help="m2 of ArcFace (default 0.5) or m3 of CosFace (default 0.35)")
+    ap.add_argument("--loss", default="ce", choices=["ce", "focal"],
+                    help="softmax cross-entropy, or the reference's focal loss gamma (1 - p)^alpha CE")
+    ap.add_argument("--focal-gamma", type=float, default=1.0, help="gamma of the focal loss: the multiplier")
+    ap.add_argument("--focal-alpha", type=float, default=2.0, help="alpha of the focal loss: the exponent")
     args = ap.parse_args()
+    loss_kind = FocalLoss(args.focal_gamma, args.focal_alpha) if args.loss == "focal" else None
     if args.margin == "arcface":
         margin = AdditiveMargin.arcface(args.scale, 0.5 if args.margin_value is None else args.margin_value)
     elif args.margin == "cosface":
@@ -121,7 +127,7 @@ def main():
         from tf_face_toolbox_b200 import ShardedASoftmaxHead
         head = ShardedASoftmaxHead(512, args.classes, m=4, mode=args.mode, device=dev, lambda_state=lam,
                                    transport=args.transport, batch_global=args.batch,   # N(0, 0.001) shards
-                                   margin=margin)
+                                   margin=margin, loss=loss_kind)
 
         def head_call(feats, labels):
             loss, dX, _ = head.step(feats, labels, optimizer=opt_head)                  # lambda from the clock
@@ -131,7 +137,8 @@ def main():
 
         def head_call(feats, labels):
             loss, _, dX, _ = asoftmax_head(feats, labels, args.classes, 4, lam.step(),
-                                           weights=W, mode=args.mode, optimizer=opt_head, margin=margin)
+                                           weights=W, mode=args.mode, optimizer=opt_head, margin=margin,
+                                           loss=loss_kind)
             return loss, dX
     # a fixed synthetic "dataset" of 4 batches so the loss can actually go down; every rank draws
     # the same global batch and keeps its slice (data_parallel.py:206-207)
@@ -152,7 +159,8 @@ def main():
         losses.append(loss)
         if rank == 0 and (step % 5 == 0 or step == args.steps - 1):
             extra = f"  lambda {lam.value():.2f}" if margin is None else f"  {args.margin} s={margin.s:g}"
-            print(f"step {step:4d}  cross_entropy {float(loss):.4f}{extra}", flush=True)
+            name = "focal_loss" if loss_kind is not None else "cross_entropy"
+            print(f"step {step:4d}  {name} {float(loss):.4f}{extra}", flush=True)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     first, last = float(torch.stack(losses[:4]).mean()), float(torch.stack(losses[-4:]).mean())

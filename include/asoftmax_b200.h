@@ -212,7 +212,7 @@ int asm_p2p_status(asm_head* h, void* cuda_stream);
  * the softmax-gradient offset, the weight-decay term in the dW epilogue's per-class coefficient)
  * and, when reg_loss_out is not NULL, writes  weight_decay/2 * sum over this shard's classes of
  * |w_j|^2  to that device float (the column sums of squares are a by-product of the norm kernel;
- * deterministic).  loss_out stays the unscaled cross-entropy.  Defaults: 1, 0, NULL.  With a
+ * deterministic).  loss_out stays the unscaled loss (asm_set_loss).  Defaults: 1, 0, NULL.  With a
  * fused optimizer armed the optimizer's own weight_decay applies instead of this one.
  */
 int asm_set_gradient_transform(asm_head* h, float grad_scale, float weight_decay, float* reg_loss_out);
@@ -246,6 +246,29 @@ typedef struct {
   float   s, m2, m3;
 } asm_margin;
 int asm_set_margin(asm_head* h, const asm_margin* margin);
+
+/*
+ * Loss applied to the head's logits f (the margin logits of whichever margin is set), per handle;
+ * like the margin it applies to every step call and is captured with them into a CUDA graph.
+ *   ASM_LOSS_SOFTMAX_CE (default)  L = mean_i (lse_i - f_iy), the softmax cross-entropy.
+ *   ASM_LOSS_FOCAL                 L = mean_i gamma (1 - p_iy)^alpha (lse_i - f_iy),
+ *                                  p_iy = softmax(f_i)_{y_i}: the reference's focal_loss (loss.py).
+ *                                  The names follow the reference, not Lin et al.: gamma is the
+ *                                  multiplier and alpha the exponent.  The gradient differentiates
+ *                                  through (1 - p)^alpha (no stop-gradient): every row's softmax
+ *                                  gradient is multiplied by
+ *                                  w_i = gamma ((1 - p)^alpha + alpha p (1 - p)^(alpha - 1) ce_i).
+ * loss_out (asm_forward included) receives the loss selected here; grad_scale, weight_decay and
+ * reg_loss_out (asm_set_gradient_transform) apply to it as to the cross-entropy.  loss == NULL
+ * restores the default.  gamma must be finite and > 0, alpha finite and >= 0; anything else returns
+ * ASM_ERR_INVALID_ARG and changes nothing.
+ */
+enum { ASM_LOSS_SOFTMAX_CE = 0, ASM_LOSS_FOCAL = 1 };
+typedef struct {
+  int32_t kind;
+  float   gamma, alpha;
+} asm_loss;
+int asm_set_loss(asm_head* h, const asm_loss* loss);
 
 /* CUDA-graph support.  Kernel arguments are frozen when a step is captured into a graph, so
  * lambda (which anneals per step) can instead be read from a caller-owned DEVICE float:

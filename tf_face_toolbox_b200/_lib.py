@@ -52,6 +52,13 @@ class AsmMargin(C.Structure):
 MARGIN_ASOFTMAX, MARGIN_ADDITIVE = 0, 1
 
 
+class AsmLoss(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("gamma", C.c_float), ("alpha", C.c_float)]
+
+
+LOSS_SOFTMAX_CE, LOSS_FOCAL = 0, 1
+
+
 class AsmError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"asoftmax_b200 error {code}: {msg}")
@@ -84,6 +91,7 @@ SYMBOLS = {
     "asm_set_gradient_transform": (C.c_int, [_P, C.c_float, C.c_float, _P]),
     "asm_set_embedding_dtype": (C.c_int, [_P, C.c_int32]),
     "asm_set_margin": (C.c_int, [_P, C.POINTER(AsmMargin)]),
+    "asm_set_loss": (C.c_int, [_P, C.POINTER(AsmLoss)]),
     "asm_set_lambda_device": (C.c_int, [_P, _P]),
     "asm_set_profiling": (C.c_int, [_P, C.c_int]),
     "asm_get_profile": (C.c_int, [_P, C.c_int32, _P, _P]),

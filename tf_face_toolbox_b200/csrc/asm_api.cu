@@ -66,7 +66,7 @@ thread_local char g_create_err[512] = "";
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct Layout {
-  size_t ylocal, flags, n, inv_n, inv_c, margin, tgt_s, tgt_f, part, stats_local, lse, negoff, gtarget, rcoef, rowloss, counter,
+  size_t ylocal, flags, n, inv_n, inv_c, margin, tgt_s, tgt_f, part, stats_local, lse, negoff, gtarget, rcoef, rowloss, rowgrad, counter,
       q_part, G, dx_part, Xb, Wb, Xs, Xg, step_dev, wsq_part, wsq_ticket, total;
   int Cp, NT, MT;
   size_t dx_capacity;
@@ -146,6 +146,7 @@ Layout make_layout(const asm_config& c, int num_sms) {
     L.Xg = take(B * D * 4);
     L.step_dev = take(256);
   }
+  L.rowgrad = take(B * 4);   // last: every buffer before it keeps the offset it had without it
   L.total = off;
   return L;
 }
@@ -489,6 +490,7 @@ int asm_create(asm_head** out, const asm_config* cfg) {
   s.gtarget = (float*)(w + L.gtarget);
   s.rcoef = (float*)(w + L.rcoef);
   s.rowloss = (float*)(w + L.rowloss);
+  s.rowgrad = (float*)(w + L.rowgrad);
   s.counter = (unsigned int*)(w + L.counter);
   s.q_part = (float*)(w + L.q_part);
   s.wsq_part = (float*)(w + L.wsq_part);
@@ -507,6 +509,7 @@ int asm_create(asm_head** out, const asm_config* cfg) {
     s.Xs = (float*)(w + L.Xs);
   }
   s.mg.kind = 0;
+  s.ls = LossParams{0, 1.0f, 0.0f};
   if (cfg->world > 1) {
     h->Xg = (float*)(w + L.Xg);
     h->p2p.step_dev = (unsigned*)(w + L.step_dev);     // zeroed with the workspace
@@ -752,6 +755,20 @@ int asm_set_margin(asm_head* h, const asm_margin* margin) {
     return fail(h, ASM_ERR_INVALID_ARG, "unknown margin kind%s", "");
   }
   h->st.mg = g;
+  return ASM_OK;
+}
+
+int asm_set_loss(asm_head* h, const asm_loss* loss) {
+  if (!h) return ASM_ERR_INVALID_ARG;
+  LossParams l{0, 1.0f, 0.0f};
+  if (loss && loss->kind == ASM_LOSS_FOCAL) {
+    if (!(isfinite(loss->gamma) && loss->gamma > 0.f) || !(isfinite(loss->alpha) && loss->alpha >= 0.f))
+      return fail(h, ASM_ERR_INVALID_ARG, "focal loss needs finite gamma > 0 and finite alpha >= 0%s", "");
+    l = LossParams{1, loss->gamma, loss->alpha};
+  } else if (loss && loss->kind != ASM_LOSS_SOFTMAX_CE) {
+    return fail(h, ASM_ERR_INVALID_ARG, "unknown loss kind%s", "");
+  }
+  h->st.ls = l;
   return ASM_OK;
 }
 

@@ -36,6 +36,13 @@ __host__ __device__ inline void opt_apply(const OptParams& o, float grad, float&
   }
 }
 
+// Loss on the logits (asm_set_loss): kind 0 = softmax cross-entropy, 1 = the reference's focal
+// loss gamma (1 - p_y)^alpha CE (gamma the multiplier, alpha the exponent; DESIGN.md section 2.2).
+struct LossParams {
+  int kind;
+  float gamma, alpha;
+};
+
 // NVLink peer-memory transport of the class-sharded step (asm_p2p.cu)
 constexpr int kMaxPeers = 8;
 constexpr int kFlagStride = 16;        // flag words per phase
@@ -138,10 +145,10 @@ struct Step {
   int NT;                    // number of column tiles of the forward kernel
   float* stats_local;        // [3, B]
   float* lse;                // [B]   M_i + log Z_i (global)
-  float* negoff;             // [B]   -(lse_i * log2 e) + log2(1/B): exp2 offset of the backward
+  float* negoff;             // [B]   -(lse_i * log2 e) + log2(gscale/B) (+ log2 w_i, focal): exp2 offset of the backward
   float* gtarget;            // [B]   G'_{i,y_i}
   float* rcoef;              // [B]   r_i  (0 if not owned)
-  float* rowloss;            // [B]   lse_i - f_{i,y}
+  float* rowloss;            // [B]   lse_i - f_{i,y}  (focal: gamma (1 - p_iy)^alpha (lse_i - f_{i,y}))
   unsigned int* counter;     // [1]   last-block-done ticket of the combine kernel
   float* q_part;             // [MT, Cp] column sums  sum_i G'_ij s_ij per 128-row group
   int MT;
@@ -168,6 +175,11 @@ struct Step {
   // patches s * phi(t) in, combine sets G'_y = g_y phi'(t) and r = 0, dx_finish projects each row.
   Margin mg;
   float* Xs;                 // [B, D] fp32 s * x_i / n_i: what the CUDA-core kernels read in place of X (additive kind)
+  // loss on the logits (asm_set_loss).  Read by the combine kernels only (row_epilogue): focal
+  // loss multiplies every row's softmax gradient by one scalar w_i, which rides in negoff, gtarget,
+  // rcoef and rowgrad, so no GEMM kernel sees it.
+  LossParams ls;
+  float* rowgrad;            // [B]   invB * gscale * w_i: the CUDA-core recompute's per-row gradient factor
 };
 
 // prep: column norms of W (+ bf16 copy), row norms of X (+ bf16 copy), label localisation.

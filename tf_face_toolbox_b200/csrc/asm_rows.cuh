@@ -15,6 +15,24 @@ namespace asmh {
 // dx_finish_rows_margin replaces the r_i x_i term).
 // A row whose label lies outside [0, C_total) (ylocal == -2) has no defined loss: it gets NaN,
 // as the reference's sparse_softmax_cross_entropy does on the GPU (nets/sphere.py:109).
+//
+// Focal loss (s.ls.kind == 1, DESIGN.md section 2.2): with ce = lse - f_y, p = e^{-ce}, u = 1 - p,
+//   loss_i = gamma u^alpha ce,   d loss_i / d f_ij = w_i (softmax_ij - delta_{j,y_i}),
+//   w_i = gamma (u^alpha + alpha p (ce / u) u^alpha)        (ce / u := 1 at u == 0)
+// so the row's whole gradient is the cross-entropy one times w_i: log2 w_i joins the exp2 offset,
+// G'_y and r are multiplied by it.  w_i depends only on the global (M, Z, f_y), so every class
+// shard computes the same value.  w_i = 0 (ce == 0, alpha > 0) gives negoff = -inf, which the
+// recompute kernels turn into exp2(-inf) = 0.
+__device__ __forceinline__ void focal_row(const LossParams& ls, float ce, float& w, float& loss) {
+  const float c = fmaxf(ce, 0.f);                // rounding can leave lse a hair below f_y
+  const float p = expf(-c);
+  const float u = -expm1f(-c);                   // 1 - p without cancellation
+  const float ua = powf(u, ls.alpha);            // powf(u, 0) == 1: alpha = 0 gives w = gamma exactly
+  const float cu = u > 0.f ? c / u : 1.0f;
+  w = ls.gamma * (ua + ls.alpha * p * cu * ua);
+  loss = ls.gamma * ua * ce;
+}
+
 __device__ __forceinline__ void row_epilogue(const Step& s, int row, float m, float z, float fy,
                                              int yl_row, float tgt_f_row, float tgt_s_row,
                                              float inv_n_row) {
@@ -22,8 +40,16 @@ __device__ __forceinline__ void row_epilogue(const Step& s, int row, float m, fl
   const float lse = m + logf(z);
   s.lse[row] = lse;
   const float gB = s.invB * s.gscale;            // every gradient carries 1/B and the caller's scale
-  s.negoff[row] = -lse * 1.4426950408889634f + log2f(gB);
-  s.rowloss[row] = yl_row == -2 ? __int_as_float(0x7fc00000) : lse - fy;
+  float negoff = -lse * 1.4426950408889634f + log2f(gB);
+  float loss = lse - fy, w = 1.0f;
+  const bool focal = s.ls.kind != 0;
+  if (focal) {
+    focal_row(s.ls, loss, w, loss);
+    negoff += log2f(w);
+  }
+  s.negoff[row] = negoff;
+  s.rowgrad[row] = focal ? gB * w : gB;
+  s.rowloss[row] = yl_row == -2 ? __int_as_float(0x7fc00000) : loss;
   float gt = 0.f, r = 0.f;
   if (owned && s.mg.kind != 0) {                 // additive: G'_y = g_y phi'(t), r = 0
     float phi, dphi;
@@ -38,6 +64,10 @@ __device__ __forceinline__ void row_epilogue(const Step& s, int row, float m, fl
     const float il = 1.0f / (1.0f + lam);
     gt = gy * (lam + dpsi) * il;
     r = gy * (psi - t * dpsi) * il * inv_n_row;
+  }
+  if (focal) {
+    gt *= w;
+    r *= w;
   }
   s.gtarget[row] = gt;
   s.rcoef[row] = r;

@@ -6,7 +6,8 @@
 // fully predicated loads, so there is no padding or alignment requirement in fp32 mode.
 //   FWD  : S = X . W            epilogue: scale by 1/c_j, margin on the target column,
 //                               per-row (max, sumexp) partial per column tile (+ logits)
-//   BWDG : S recomputed         epilogue: G'' = G' / c_j  (fp32, [B,Cp]) and the column
+//   BWDG : S recomputed         epilogue: G'' = G' / c_j  (fp32, [B,Cp]; the non-target G'
+//                               carries the per-row factor rowgrad = gscale w_i / B) and the column
 //                               sums q_j = sum_i G'_ij s_ij per 128-row tile
 //   DW   : dWhat'' = X^T . G''  epilogue: dW = dWhat'' - W * q_j / c_j^2
 //   DX   : dX partial = G'' . W^T over a K-split of the classes
@@ -209,13 +210,14 @@ __global__ void __launch_bounds__(256) simt_kernel(Step s, int k_per_split) {
         const int yl = s.ylocal[i];
         const float lse = s.lse[i];
         const float gt = s.gtarget[i];
+        const float gB = s.rowgrad[i];        // invB * gscale * w_i (exactly invB for CE at gscale 1)
 #pragma unroll
         for (int b = 0; b < 8; ++b) {
           const int j = n0 + sub_index(tx, b);
           if (j < s.Cp) {
             const float sv = acc[a][b] * ic[b];
             float gp = 0.f;
-            if (j < s.C) gp = (j == yl) ? gt : __expf(sv - lse) * s.invB;
+            if (j < s.C) gp = (j == yl) ? gt : __expf(sv - lse) * gB;
             cs[b] = fmaf(gp, sv, cs[b]);
             Gw[(size_t)i * s.Cp + j] = gp * ic[b];
           }

@@ -85,6 +85,25 @@ class AdditiveMargin:
         return _lib.AsmMargin(_lib.MARGIN_ADDITIVE, self.s, self.m2, self.m3)
 
 
+# --------------------------------------------------------------------------------------
+# focal loss (loss.py:18-27 of the reference) in place of the softmax cross-entropy
+# --------------------------------------------------------------------------------------
+@dataclass(frozen=True)
+class FocalLoss:
+    """The reference's focal_loss on the head's (margin) logits f:
+    L = mean_i gamma * (1 - p_iy)^alpha * (lse_i - f_iy), p_iy = softmax(f_i)[y_i].
+    The names follow the reference, not Lin et al.: gamma is the multiplier and alpha the
+    exponent (the paper calls them the other way round).  The gradient goes through the
+    modulating factor (1 - p)^alpha; it is not a stop-gradient.  gamma=1, alpha=0 is the plain
+    cross-entropy.  Pass it as `loss=` to the head's entry points (None: cross-entropy).
+    gamma > 0 and alpha >= 0, both finite, are checked by the library."""
+    gamma: float = 1.0
+    alpha: float = 2.0
+
+    def _struct(self) -> "_lib.AsmLoss":
+        return _lib.AsmLoss(_lib.LOSS_FOCAL, self.gamma, self.alpha)
+
+
 def _as_lambda(lambda_state) -> float:
     if lambda_state is None:
         return 0.0
@@ -94,12 +113,12 @@ def _as_lambda(lambda_state) -> float:
 
 
 # --------------------------------------------------------------------------------------
-# handle cache: one asm_head per (device, shard geometry, B_max, m, mode, margin)
+# handle cache: one asm_head per (device, shard geometry, B_max, m, mode, margin, loss)
 # --------------------------------------------------------------------------------------
 class _Handle:
     def __init__(self, device: torch.device, D: int, C_total: int, C_local: int, class_offset: int,
                  B_max: int, m: int, mode: str, rank: int = 0, world: int = 1,
-                 margin: Optional[AdditiveMargin] = None):
+                 margin: Optional[AdditiveMargin] = None, loss: Optional[FocalLoss] = None):
         self.lib = _lib.load()
         if device.type != "cuda":
             raise RuntimeError("the A-softmax head runs on a CUDA (B200) device only; no CPU fallback")
@@ -114,6 +133,13 @@ class _Handle:
         if margin is not None:
             # set once: the margin is part of the handle-cache key, never switched per call
             rc = self.lib.asm_set_margin(self.ptr, C.byref(margin._struct()))
+            if rc != _lib.ASM_OK:
+                err = _lib.AsmError(rc, (self.lib.asm_last_error(self.ptr) or b"").decode())
+                self.close()
+                raise err
+        if loss is not None:
+            # likewise part of the key
+            rc = self.lib.asm_set_loss(self.ptr, C.byref(loss._struct()))
             if rc != _lib.ASM_OK:
                 err = _lib.AsmError(rc, (self.lib.asm_last_error(self.ptr) or b"").decode())
                 self.close()
@@ -144,7 +170,7 @@ def _round_batch(B: int) -> int:
 
 
 def get_handle(device, D, C_total, C_local, class_offset, B, m, mode, rank=0, world=1, tag=None,
-               margin: Optional[AdditiveMargin] = None) -> _Handle:
+               margin: Optional[AdditiveMargin] = None, loss: Optional[FocalLoss] = None) -> _Handle:
     """`tag` separates handles with different per-handle state (e.g. a CUDA-graph step that
     reads lambda from device memory) from the plain eager ones."""
     device = torch.device(device)
@@ -152,10 +178,12 @@ def get_handle(device, D, C_total, C_local, class_offset, B, m, mode, rank=0, wo
         device = torch.device("cuda", torch.cuda.current_device())
     if margin is not None and not isinstance(margin, AdditiveMargin):
         raise TypeError("margin must be None (A-softmax) or an AdditiveMargin")
-    key = (device.index, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin, tag)
+    if loss is not None and not isinstance(loss, FocalLoss):
+        raise TypeError("loss must be None (softmax cross-entropy) or a FocalLoss")
+    key = (device.index, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin, loss, tag)
     h = _HANDLES.get(key)
     if h is None:
-        h = _Handle(device, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin)
+        h = _Handle(device, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin, loss)
         h.key = key
         _HANDLES[key] = h
         untagged = [k for k in _HANDLES if k[-1] is None]
@@ -240,7 +268,7 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
                   check_labels: bool = False, optimizer: Optional["FusedOptimizer"] = None,
                   grad_scale: float = 1.0, weight_decay: float = 0.0,
                   reg_loss_out: Optional[torch.Tensor] = None, margin: Optional[AdditiveMargin] = None,
-                  _handle_tag=None
+                  loss: Optional[FocalLoss] = None, _handle_tag=None
                   ) -> Tuple[torch.Tensor, Optional[torch.Tensor], Optional[torch.Tensor], Optional[torch.Tensor]]:
     """A-softmax head forward + backward on one GPU that owns every class.
 
@@ -256,9 +284,12 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
     gradients without a single extra pass over [D, C]: dX, dW come back multiplied by grad_scale
     (mult_lr / num_gpus, data_parallel.py:37), dW includes weight_decay * W (the gradient of
     reg_loss, nets/sphere.py:88) and reg_loss_out (a 1-element CUDA float tensor) receives
-    weight_decay/2 * |W|^2 (nets/net_base.py:103-107).  The returned loss is the plain cross-entropy.
+    weight_decay/2 * |W|^2 (nets/net_base.py:103-107).  The returned loss is the unscaled loss
+    without reg_loss.
     `margin` (an AdditiveMargin) selects the ArcFace / CosFace head on normalised embeddings
     instead of A-softmax; `m` and lambda_state are then ignored.  None: A-softmax.
+    `loss` (a FocalLoss) replaces the softmax cross-entropy by the reference's focal loss on the
+    same logits; loss, dX and dW are then those of the focal loss.  None: cross-entropy.
     Asynchronous on the current CUDA stream.
     """
     _check_inputs(embeddings, labels, weights, num_classes)
@@ -271,9 +302,9 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
     y = labels.contiguous()
     B, D = X.shape
     Cn = W.shape[1]
-    h = get_handle(X.device, D, Cn, Cn, 0, B, m, mode, tag=_handle_tag, margin=margin)
+    h = get_handle(X.device, D, Cn, Cn, 0, B, m, mode, tag=_handle_tag, margin=margin, loss=loss)
     lam = _as_lambda(lambda_state)
-    loss = torch.empty(1, device=X.device, dtype=torch.float32)
+    loss_out = torch.empty(1, device=X.device, dtype=torch.float32)
     logits = torch.empty(B, Cn, device=X.device, dtype=torch.float32) if return_logits else None
     stream = C.c_void_p(torch.cuda.current_stream(X.device).cuda_stream)
     transform = grad_scale != 1.0 or weight_decay != 0.0 or reg_loss_out is not None
@@ -295,7 +326,7 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
             try:
                 rc = h.lib.asm_forward_backward(
                     h.ptr, X.data_ptr(), B, y.data_ptr(), y.element_size(), W.data_ptr(), lam,
-                    loss.data_ptr(), logits.data_ptr() if logits is not None else None,
+                    loss_out.data_ptr(), logits.data_ptr() if logits is not None else None,
                     dX.data_ptr(), dW.data_ptr() if dW is not None else None, stream)
             finally:
                 if optimizer is not None:
@@ -304,7 +335,7 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
             dX = dW = None
             rc = h.lib.asm_forward(
                 h.ptr, X.data_ptr(), B, y.data_ptr(), y.element_size(), W.data_ptr(), lam,
-                loss.data_ptr(), logits.data_ptr() if logits is not None else None, stream)
+                loss_out.data_ptr(), logits.data_ptr() if logits is not None else None, stream)
         if transform:
             h.lib.asm_set_gradient_transform(h.ptr, 1.0, 0.0, None)     # the handle is shared: back to defaults
         if x16:
@@ -312,7 +343,7 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
         _lib.check(rc, h.ptr)
         if check_labels:
             _lib.check(h.lib.asm_check_labels(h.ptr, stream), h.ptr)
-    return loss[0], logits, dX, dW
+    return loss_out[0], logits, dX, dW
 
 
 def last_launch_count(device, D, C_total, B, m, mode) -> int:
@@ -336,7 +367,8 @@ class GraphedASoftmaxStep:
     """
 
     def __init__(self, weights: torch.Tensor, batch_size: int, m: int = 4, mode: str = "bf16",
-                 labels_dtype=torch.int32, margin: Optional[AdditiveMargin] = None):
+                 labels_dtype=torch.int32, margin: Optional[AdditiveMargin] = None,
+                 loss: Optional[FocalLoss] = None):
         assert weights.is_cuda and weights.dtype == torch.float32 and weights.is_contiguous()
         dev = weights.device
         self.W = weights
@@ -345,9 +377,9 @@ class GraphedASoftmaxStep:
         self.y = torch.zeros(batch_size, device=dev, dtype=labels_dtype)
         self.lam = torch.zeros(1, device=dev, dtype=torch.float32)
         self._lam_host = torch.zeros(1, dtype=torch.float32).pin_memory()
-        self.m, self.mode, self.Cn, self.margin = m, mode, Cn, margin
+        self.m, self.mode, self.Cn, self.margin, self.loss_kind = m, mode, Cn, margin, loss
         self._tag = ("graph", id(self))
-        h = get_handle(dev, D, Cn, Cn, 0, batch_size, m, mode, tag=self._tag, margin=margin)
+        h = get_handle(dev, D, Cn, Cn, 0, batch_size, m, mode, tag=self._tag, margin=margin, loss=loss)
         self._key = h.key
         _lib.check(h.lib.asm_set_lambda_device(h.ptr, self.lam.data_ptr()), h.ptr)
         cur = torch.cuda.current_stream(dev)
@@ -364,7 +396,8 @@ class GraphedASoftmaxStep:
 
     def _run(self):
         loss, _, dX, dW = asoftmax_head(self.X, self.y, self.Cn, self.m, 0.0, weights=self.W,
-                                        mode=self.mode, margin=self.margin, _handle_tag=self._tag)
+                                        mode=self.mode, margin=self.margin, loss=self.loss_kind,
+                                        _handle_tag=self._tag)
         return loss, dX, dW
 
     def close(self):
@@ -394,27 +427,29 @@ class GraphedASoftmaxStep:
 # torch autograd bridge: lets a torch backbone train through the fused head
 # --------------------------------------------------------------------------------------
 class ASoftmaxLoss(torch.autograd.Function):
-    """loss = ASoftmaxLoss.apply(embeddings, weights, labels, m, lam, mode[, upstream[, margin]]).  The fused
+    """loss = ASoftmaxLoss.apply(embeddings, weights, labels, m, lam, mode[, upstream[, margin[, loss]]]).  The fused
     call already produced dX and dW, so backward only hands them on.  `upstream` (a float) is the
     gradient the caller promises to send into this loss (1.0 for a plain `loss.backward()`, the loss
     scale otherwise): it is applied inside the kernels and backward returns the stored gradients
     untouched -- no pass over [D, C].  Without it backward multiplies by the incoming gradient.
-    `margin` (an AdditiveMargin, or None for A-softmax) as in asoftmax_head."""
+    `margin` (an AdditiveMargin, or None for A-softmax) and `loss` (a FocalLoss, or None for the
+    cross-entropy) as in asoftmax_head."""
 
     @staticmethod
-    def forward(ctx, embeddings, weights, labels, m, lam, mode, upstream=None, margin=None):
-        loss, _, dX, dW = asoftmax_head(embeddings, labels, weights.shape[1], m, lam, weights=weights, mode=mode,
-                                        grad_scale=1.0 if upstream is None else float(upstream), margin=margin)
+    def forward(ctx, embeddings, weights, labels, m, lam, mode, upstream=None, margin=None, loss=None):
+        value, _, dX, dW = asoftmax_head(embeddings, labels, weights.shape[1], m, lam, weights=weights, mode=mode,
+                                         grad_scale=1.0 if upstream is None else float(upstream), margin=margin,
+                                         loss=loss)
         ctx.save_for_backward(dX, dW)
         ctx.upstream = upstream
-        return loss
+        return value
 
     @staticmethod
     def backward(ctx, grad_out):
         dX, dW = ctx.saved_tensors
         if ctx.upstream is not None:
-            return dX, dW, None, None, None, None, None, None
-        return grad_out * dX, grad_out * dW, None, None, None, None, None, None
+            return dX, dW, None, None, None, None, None, None, None
+        return grad_out * dX, grad_out * dW, None, None, None, None, None, None, None
 
 
 # --------------------------------------------------------------------------------------
@@ -435,7 +470,8 @@ class ASoftmaxHead:
     def __init__(self, num_features: int, num_classes: int, m: int = 4, weight_decay: float = 5e-4,
                  mode: str = "bf16", device="cuda", lambda_state: Optional[LambdaState] = None,
                  return_logits: bool = False, seed: Optional[int] = None, num_gpus: int = 1,
-                 mult_lr: float = 1.0, margin: Optional[AdditiveMargin] = None):
+                 mult_lr: float = 1.0, margin: Optional[AdditiveMargin] = None,
+                 loss: Optional[FocalLoss] = None):
         gen = None
         if seed is not None:
             gen = torch.Generator(device="cpu").manual_seed(seed)
@@ -445,6 +481,7 @@ class ASoftmaxHead:
         self.num_classes = num_classes
         self.m = m
         self.margin = margin                         # None: A-softmax; AdditiveMargin: ArcFace / CosFace
+        self.loss = loss                             # None: cross-entropy; FocalLoss: loss.py's focal_loss
         self.weight_decay = weight_decay
         self.mode = mode
         self.lambda_state = lambda_state if lambda_state is not None else LambdaState()
@@ -467,7 +504,7 @@ class ASoftmaxHead:
                                              weights=self.weights, mode=self.mode,
                                              return_logits=self.return_logits, grad_scale=scale,
                                              weight_decay=self.weight_decay, reg_loss_out=self._reg,
-                                             margin=self.margin)
+                                             margin=self.margin, loss=self.loss)
         self._last = dict(loss=loss, dX=dX, dW=dW, lam=lam, scale=scale, reg=self._reg[0].clone())
         out = {"logits": logits, "features": features}
         return out
@@ -476,7 +513,7 @@ class ASoftmaxHead:
     def loss_function(self, scope, labels, **logits):
         assert self._last is not None, "forward(...) must run first"
         losses = [self._last["loss"]]
-        losses_name = ["cross_entropy"]
+        losses_name = ["focal_loss" if self.loss is not None else "cross_entropy"]
         # _regularize (nets/net_base.py:103-107): contrib l2_regularizer = wd * sum(w^2)/2, a
         # by-product of the norm kernel's column sums (no pass over W here)
         losses.append(self._last["reg"])
@@ -487,7 +524,7 @@ class ASoftmaxHead:
         return losses, losses_name, others
 
     def gradients(self, num_gpus: Optional[int] = None, mult_lr: Optional[float] = None):
-        """(dX, dW) of total_loss = cross_entropy + reg_loss, scaled like _grad_var
+        """(dX, dW) of total_loss = cross_entropy (or focal_loss) + reg_loss, scaled like _grad_var
         (data_parallel.py:37): both came out of the kernels in that form (dW includes wd * W).
         Asking for a scale other than the configured one rescales them (one eager pass)."""
         want = (self.mult_lr if mult_lr is None else mult_lr) / (self.num_gpus if num_gpus is None else num_gpus)

@@ -24,7 +24,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .head import AdditiveMargin, LambdaState, _as_lambda, get_handle
+from .head import AdditiveMargin, FocalLoss, LambdaState, _as_lambda, get_handle
 
 
 def shard_bounds(num_classes: int, world: int, rank: int) -> Tuple[int, int]:
@@ -36,9 +36,9 @@ def shard_bounds(num_classes: int, world: int, rank: int) -> Tuple[int, int]:
 class _CudaShard:
     """Per-shard compute through the C ABI (asm_forward_partial / asm_backward_partial)."""
 
-    def __init__(self, D, C_total, lo, hi, m, mode, rank, world, device, margin=None):
+    def __init__(self, D, C_total, lo, hi, m, mode, rank, world, device, margin=None, loss=None):
         self.args = (D, C_total, hi - lo, lo, m, mode, rank, world)
-        self.margin = margin
+        self.margin, self.loss = margin, loss
         self.device = torch.device(device)
         # a handle carries per-step state (the pointers of the step in flight, an armed optimizer):
         # every shard object gets its own instead of sharing one with same-shaped callers
@@ -48,7 +48,7 @@ class _CudaShard:
     def _handle(self, B):
         D, C_total, C_local, lo, m, mode, rank, world = self.args
         h = get_handle(self.device, D, C_total, C_local, lo, B, m, mode, rank, world, tag=self.tag,
-                       margin=self.margin)
+                       margin=self.margin, loss=self.loss)
         if self.lambda_dev is not None:
             _lib.check(h.lib.asm_set_lambda_device(h.ptr, self.lambda_dev.data_ptr()), h.ptr)
         return h
@@ -93,13 +93,17 @@ class ShardedASoftmaxHead:
                  device="cuda", group=None, lambda_state: Optional[LambdaState] = None,
                  weights_full: Optional[torch.Tensor] = None, seed: int = 0, shard_compute=None,
                  transport: str = "nccl", batch_global: Optional[int] = None,
-                 weights_shard: Optional[torch.Tensor] = None, margin: Optional[AdditiveMargin] = None):
-        """`margin` (an AdditiveMargin) selects the ArcFace / CosFace head; None: A-softmax.  An
-        injected `shard_compute` is given the margin through its own constructor."""
+                 weights_shard: Optional[torch.Tensor] = None, margin: Optional[AdditiveMargin] = None,
+                 loss: Optional[FocalLoss] = None):
+        """`margin` (an AdditiveMargin) selects the ArcFace / CosFace head; None: A-softmax.
+        `loss` (a FocalLoss) replaces the cross-entropy by the focal loss on both transports;
+        None: cross-entropy.  An injected `shard_compute` is given the margin and the loss
+        through its own constructor."""
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.D, self.C, self.m, self.mode, self.margin = num_features, num_classes, m, mode, margin
+        self.loss = loss
         self.lo, self.hi = shard_bounds(num_classes, self.world, self.rank)
         if self.hi <= self.lo:
             raise ValueError("more ranks than classes: empty shard")
@@ -116,7 +120,7 @@ class ShardedASoftmaxHead:
         self.weights = w.contiguous().to(self.device)            # [D, C_local]
         self.lambda_state = lambda_state if lambda_state is not None else LambdaState()
         self.compute = shard_compute if shard_compute is not None else _CudaShard(
-            num_features, num_classes, self.lo, self.hi, m, mode, self.rank, self.world, self.device, margin)
+            num_features, num_classes, self.lo, self.hi, m, mode, self.rank, self.world, self.device, margin, loss)
         # transport "nvlink": no NCCL in the step -- the library's kernels read the peers'
         # symmetric buffers over NVLink (asm_step_p2p).  Needs the global batch up front.
         self.transport = transport
@@ -153,7 +157,7 @@ class ShardedASoftmaxHead:
         import torch.distributed._symmetric_memory as symm_mem
         D, C_total, C_local, lo, m, mode, rank, world = self.compute.args
         h = get_handle(self.device, D, C_total, C_local, lo, batch_global, m, mode, rank, world,
-                       tag=(tag, id(self)), margin=self.margin)
+                       tag=(tag, id(self)), margin=self.margin, loss=self.loss)
         nbytes = int(h.lib.asm_p2p_bytes(C.byref(h.cfg)))
         if nbytes == 0:
             raise RuntimeError("asm_p2p_bytes: unsupported configuration (2..8 ranks)")
@@ -203,7 +207,7 @@ class ShardedASoftmaxHead:
         `center` = dict(centers=[C_local, D] shard, alpha=.., weight=..) adds the class-sharded
         center loss (loss.py:29-45) on the same gathered batch: the shard's centers are updated in
         place, its gradient joins the dX contribution before the reduce-scatter, and the returned
-        loss becomes (cross_entropy, center_loss summed over the shards).  Host-collective
+        loss becomes (cross_entropy or focal loss, center_loss summed over the shards).  Host-collective
         transport only."""
         lam = _as_lambda(lambda_state) if lambda_state is not None else self.lambda_state.step()
         if self._p2p is not None:
@@ -264,7 +268,7 @@ class ShardedASoftmaxHead:
         # from the device scalar; the eager step() keeps its own by-value handle
         eager_compute = self.compute
         gcompute = _CudaShard(self.D, self.C, self.lo, self.hi, self.m, self.mode, self.rank,
-                              self.world, self.device, self.margin)
+                              self.world, self.device, self.margin, self.loss)
         gcompute.tag = ("graph", id(self))
         gcompute.lambda_dev = self._glam
         self.compute = gcompute
