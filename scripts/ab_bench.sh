@@ -1,6 +1,7 @@
 # same-box A/B of an environment knob: bash scripts/ab_bench.sh VAR "v1 v2 ..." [bench args]
 mkdir -p gpurun_out
-VAR=${1:-ASM_UMMA_DEBUG}; VALS=${2:-"0 8"}; shift 2
+USAGE='usage: bash scripts/ab_bench.sh VAR "v1 v2 ..." [bench args]'
+VAR=${1:?$USAGE}; VALS=${2:?$USAGE}; shift 2
 for rep in 1 2; do
 for v in $VALS; do
   env $VAR=$v timeout 100 python bench.py --no-cpu-baseline --steps 100 --warmup 5 "$@" 2>/dev/null | tail -1 > gpurun_out/ab_$v.json

@@ -114,11 +114,6 @@ OPT_VARIANTS = {
 
 # knobs read by the library that this module does not vary, and why
 EXCLUDED = {
-    "ASM_UMMA_MN_LBO": "bring-up only: a wrong descriptor faults by design",
-    "ASM_UMMA_MN_SBO": "bring-up only: a wrong descriptor faults by design",
-    "ASM_UMMA_MN_KSTEP": "bring-up only: a wrong descriptor faults by design",
-    "ASM_UMMA_DEBUG": "bring-up only: work-skipping bits, refused by the product build",
-    "ASM_L2_PERSIST_MB": "changes the device-wide persisting-L2 limit, a setting shared with other processes",
     "ASM_P2P_TIMEOUT_MS": "NVLink transport, covered by test_p2p_gpu.py",
     "ASM_P2P_WAITERS": "NVLink transport, covered by test_p2p_gpu.py",
     "ASM_MAX_HANDLES": "size of the Python handle cache, no kernel path",

@@ -11,8 +11,8 @@ import os
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# ASM_B200_LIB selects another build of the same library (the -DASM_BRINGUP one under lib/bringup/,
-# for kernel bring-up experiments only; bench.py reports any ASM_* variable in its JSON line)
+# ASM_B200_LIB selects another build of the same library (the `make TIMING=1` one under lib/timing/,
+# or a build of another commit for an A/B run; bench.py reports any ASM_* variable in its JSON line)
 LIB_PATH = os.environ.get("ASM_B200_LIB") or os.path.join(_HERE, "lib", "libasoftmax_b200.so")
 CSRC = os.path.join(_HERE, "csrc")
 

@@ -31,7 +31,7 @@ struct asm_head {
   float* dw_scratch = nullptr;   // [D, C_local] fp32, allocated on first use of opt_stream
   bool defer_loss = true;        // ASM_DEFER_LOSS=0: combine reduces the loss itself (A/B knob)
   bool tc = false;               // tcgen05 kernels (bf16 mode, or fp32 mode through bf16 planes)
-  UmmaTuning tune{8192, 1024, 2048, 15, 0, 0, 1, 1, 0, 3};   // CTA pairs on all four kernels (ASM_UMMA_CG=0: single-CTA)
+  UmmaTuning tune{15, 0, 1, 1, 0, 3};   // CTA pairs on all four kernels (ASM_UMMA_CG=0: single-CTA)
   bool fwd_valid = false;
   // dX branch of the backward (DX + dx_finish) runs on a second stream so that it fills the
   // SMs the DW kernel's tail leaves idle; both only depend on G'' from the BWDG kernel
@@ -45,9 +45,6 @@ struct asm_head {
   P2P p2p{};
   bool p2p_ready = false;
   float* Xg = nullptr;           // [B_max, D] gathered embeddings
-  size_t l2_persist_bytes = 0;   // ASM_L2_PERSIST_MB: pin the bf16 weight copy in L2
-  cudaStream_t l2_stream = nullptr;
-  bool l2_set = false;
   int launches = 0;
   // optional per-kernel timing (asm_set_profiling): event i is recorded before kernel i
   bool profiling = false;
@@ -239,22 +236,6 @@ int run_forward(asm_head* h, const float* X, int B, const void* labels, int labe
     s.pdl = (h->pdl && !h->profiling && cs == cudaStreamCaptureStatusNone) ? 1 : 0;
   }
   h->fwd_valid = false;
-  if (h->l2_persist_bytes && h->cfg.mode == ASM_MODE_BF16 && (!h->l2_set || h->l2_stream != stream)) {
-    // keep the bf16 operand copy of W (read by four kernels per step) resident in L2
-    cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, h->l2_persist_bytes);
-    cudaStreamAttrValue av{};
-    const size_t wb_bytes = (size_t)s.D * s.Cp * 2;
-    av.accessPolicyWindow.base_ptr = (void*)s.Wb;
-    av.accessPolicyWindow.num_bytes = wb_bytes;
-    av.accessPolicyWindow.hitRatio =
-        wb_bytes <= h->l2_persist_bytes ? 1.0f : (float)h->l2_persist_bytes / (float)wb_bytes;
-    av.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    av.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    if (cudaStreamSetAttribute(stream, cudaStreamAttributeAccessPolicyWindow, &av) != cudaSuccess)
-      cudaGetLastError();
-    h->l2_set = true;
-    h->l2_stream = stream;
-  }
   if (h->tc) {
     if ((B + 127) / 128 > h->num_sms)
       return fail(h, ASM_ERR_INVALID_ARG, "batch too large for the tcgen05 forward grid%s", "");
@@ -413,19 +394,6 @@ int asm_create(asm_head** out, const asm_config* cfg) {
   h->num_sms = sms > 0 ? sms : 148;
   h->err[0] = 0;
   const char* e;
-  if ((e = getenv("ASM_UMMA_MN_LBO"))) h->tune.mn_lbo = (uint32_t)atoi(e);
-  if ((e = getenv("ASM_UMMA_MN_SBO"))) h->tune.mn_sbo = (uint32_t)atoi(e);
-  if ((e = getenv("ASM_UMMA_MN_KSTEP"))) h->tune.mn_kstep = (uint32_t)atoi(e);
-  if ((e = getenv("ASM_UMMA_DEBUG")) && atoi(e) != 0) {
-#ifdef ASM_BRINGUP
-    h->tune.debug_flags = (uint32_t)atoi(e);
-#else
-    // work-skipping bring-up bits do not exist in the product build: refuse rather than ignore
-    delete h;
-    return fail(nullptr, ASM_ERR_INVALID_ARG,
-                "ASM_UMMA_DEBUG is set but this library was built without -DASM_BRINGUP%s", "");
-#endif
-  }
   if ((e = getenv("ASM_L2_ORDER"))) h->tune.l2_order = atoi(e) != 0;
   if ((e = getenv("ASM_DW_TMA"))) h->tune.dw_tma = atoi(e) != 0;
   if ((e = getenv("ASM_L2_HINTS"))) h->tune.l2_hints = (uint32_t)atoi(e);
@@ -446,7 +414,6 @@ int asm_create(asm_head** out, const asm_config* cfg) {
     cudaGetLastError();
     h->side = nullptr;
   }
-  if ((e = getenv("ASM_L2_PERSIST_MB"))) h->l2_persist_bytes = (size_t)atoi(e) << 20;
   const Layout L = make_layout(*cfg, h->num_sms);
   cudaError_t ce = cudaMalloc(&h->ws, L.total);
   if (ce != cudaSuccess) {

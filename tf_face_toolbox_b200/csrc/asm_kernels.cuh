@@ -216,7 +216,7 @@ int simt_dx_splits(int B, int D, int Cp);
 
 // bf16 (tcgen05 / TMEM / TMA) contractions with fused epilogues
 struct UmmaMaps {            // TMA descriptors over the bf16 workspace operands
-  CUtensorMap xb_k, xb_k256, xb_mn, wb_mn, wb_mn32, wb_k, wb_k128, g_k, g_mn, g_st, g_st32, wb_box;
+  CUtensorMap xb_k, xb_k256, xb_mn, wb_mn, wb_k, wb_k128, g_k, g_mn, g_st, g_st32, wb_box;
   // the caller's dW [D, C] fp32 seen as [D/2, 2C] (row pitch 8C bytes): even rows through a
   // tensor of extent {C, D/2}, odd rows through one of extent {2C, D/2} at column offset C
   CUtensorMap dw_even, dw_odd;
@@ -225,10 +225,8 @@ struct UmmaMaps {            // TMA descriptors over the bf16 workspace operands
   const void* dw_ptr;        // buffer the two maps above were encoded for (re-encoded when it changes)
   int dw_ok;                 // 0: dW cannot be addressed by TMA (odd C, misaligned base): direct stores
 };
-struct UmmaTuning {          // MN-major shared-memory descriptor parameters (bytes)
-  uint32_t mn_lbo, mn_sbo, mn_kstep;
+struct UmmaTuning {          // schedule of the tcgen05 kernels, per handle (defaults in asm_head, overridden by ASM_* knobs)
   uint32_t cg_mask;          // CTA pairs (cta_group::2) per kernel: bit0 FWD, bit1 BWDG, bit2 DW, bit3 DX
-  uint32_t debug_flags;      // bit0: skip epilogue math, bit1: DW without stores, bit2: X-resident forward variant (ASM_UMMA_DEBUG, bring-up only)
   uint32_t bn;               // tile width along N of FWD / BWDG / DW: 0 = chosen per launch from the unit count, 128, 256 (ASM_UMMA_BN)
   uint32_t l2_order;         // consecutive kernels sweep the classes in opposite directions (ASM_L2_ORDER=0 disables)
   uint32_t dw_tma;           // dW leaves through shared memory + TMA stores (ASM_DW_TMA=0: direct stores)
@@ -243,7 +241,6 @@ struct UmmaArgs {
   int segA[6], segB[6];
   uint64_t desc_hi_k, desc_hi_mn;
   uint32_t kstep_mn;
-  uint32_t debug_flags;
   int rev;                   // class tiles (or, with kstride, K blocks) in descending order
   int kstride;               // split-K: split z takes K blocks z, z + ks, ... instead of a contiguous range
   int dw_tma;                // DW: staged TMA stores (maps D / E valid)

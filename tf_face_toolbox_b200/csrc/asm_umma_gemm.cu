@@ -33,14 +33,6 @@
 #include "asm_kernels.cuh"
 #include "asm_umma.cuh"
 
-// Bring-up knobs (ASM_UMMA_DEBUG bits: skip the epilogue math, experimental kernel variants)
-// exist only in a -DASM_BRINGUP build; the default library cannot be told to skip work.
-#ifdef ASM_BRINGUP
-#define ASM_DBG(flags, bit) ((flags) & (bit))
-#else
-#define ASM_DBG(flags, bit) 0
-#endif
-
 namespace asmh {
 
 namespace {
@@ -60,32 +52,19 @@ constexpr int DSTG = 32 * 128 * 4;             // DW: one [32 d x 128 classes] f
 // the region after the barriers holds vec + stg (FWD / BWDG) or the weight-chunk ring (DW)
 constexpr int AUX_REGION = (AUX_VEC + AUX_STG) > AUX_WB ? (AUX_VEC + AUX_STG) : AUX_WB;
 constexpr float LOG2E = 1.4426950408889634f;
+// MN-major operand tiles in shared memory (asm_umma.cuh): 64-element MN chunks of BK k rows are
+// 8 KB apart (LBO), 8-k-row groups 1 KB apart (SBO), and a K = 16 MMA step advances 16 k rows
+constexpr uint32_t MN_LBO = 8192, MN_SBO = 1024, MN_KSTEP = 2048;
 
-// U_FWDR is an experimental forward kernel with the CTA's 128-row block of Xb RESIDENT in
-// shared memory (D <= 512): only the weight tiles stream (32-deep K stages, 5 of them), which
-// cuts the L2 -> SM operand traffic by a third.  Measured SLOWER than the streaming kernel
-// (55 vs 48 us at cfg 3): the pipeline is bound by bytes in flight (80 KB vs 192 KB), not by
-// L2 bandwidth.  Kept behind ASM_UMMA_DEBUG bit 2 as the record of that experiment.
 // U_DWOPT is the dW kernel with the classifier optimizer fused into its epilogue.
 // U_DWF is the dW kernel of the fp32 (x3) path: the correction term reads the fp32 weights.
-// U_BWDG1 is BWDG with the earlier geometry (6 operand stages, one staging buffer, two named
-// barriers per chunk), selectable with ASM_UMMA_DEBUG bit 3 for same-box A/B timing.
-enum { U_FWD = 0, U_BWDG = 1, U_DW = 2, U_DX = 3, U_FWDR = 4, U_DWOPT = 5, U_DWF = 6, U_BWDG1 = 7 };
+enum { U_FWD = 0, U_BWDG = 1, U_DW = 2, U_DX = 3, U_DWOPT = 5, U_DWF = 6 };
 
 // pipeline geometry per kernel kind
 // CG = 2: a CTA pair (cluster of 2, cta_group::2) computes one 256 x 256 tile; each CTA
 // stages its own 128 A rows and HALF of the B tile, so a stage is 32 KB and the ring is 6 deep.
 // BNT: tile width along N (256, or 128 for shards whose unit count does not fill the pairs)
-#ifndef ASM_FWD_EPI16
-#define ASM_FWD_EPI16 1
-#endif
-constexpr bool FWD_EPI16 = ASM_FWD_EPI16 != 0;
-#ifndef ASM_BWDG_EPI16
-#define ASM_BWDG_EPI16 1
-#endif
-constexpr bool BWDG_EPI16 = ASM_BWDG_EPI16 != 0;
 template <int KIND, int CG = 1, int BNT = BN_FULL> struct Geo {
-  static constexpr bool RES = (KIND == U_FWDR);
   // Epilogue warps.  The epilogues, not the MMAs, bound these kernels (the light dX epilogue
   // reaches 83 % of the tensor pipe, the forward one 62 %): each scheduler hosts only two
   // epilogue warps, which spend ~8 cycles per issued instruction on dependency and queue
@@ -93,9 +72,8 @@ template <int KIND, int CG = 1, int BNT = BN_FULL> struct Geo {
   // epilogue warps -- four per TMEM lane quarter, 64 accumulator columns each -- with
   // single-buffered TMEM loads (and, in the recompute kernel, one G'' staging block per warp) to
   // stay inside 96 registers and the shared memory.
-  static constexpr int EPIW = ((KIND == U_FWD && FWD_EPI16) || (KIND == U_BWDG && BWDG_EPI16)) && CG == 2 && BNT == 256 ? 16 : 8;
+  static constexpr int EPIW = (KIND == U_FWD || KIND == U_BWDG) && CG == 2 && BNT == 256 ? 16 : 8;
   static constexpr int NTHREADS = 128 + 32 * EPIW;
-  static constexpr int KB = (RES && CG == 1) ? 32 : BK;    // K elements per pipeline stage
   // weight-chunk buffers per column half (4 buffers paid for with one of the dW kernel's four
   // operand stages measured SLOWER: 83 vs 78 us at config 3)
   static constexpr int NWB = 2;
@@ -104,14 +82,13 @@ template <int KIND, int CG = 1, int BNT = BN_FULL> struct Geo {
   static constexpr bool DW_TMA = (KIND == U_DW && CG == 2);
   // the BWDG kernel of a CTA pair trades its 6th operand stage for double-buffered G'' staging
   static constexpr int NSB = (KIND == U_BWDG && CG == 2) ? 2 : 1;   // G'' staging buffers per column half
-  static constexpr int NST = RES ? 5 : (CG == 2 ? (DW_TMA ? 4 : (KIND == U_BWDG ? 5 : 6)) : STAGES);   // pipeline depth
-  static constexpr int A_ST = RES ? 0 : BM * KB * 2;       // A bytes per stage
-  static constexpr int B_ST = BNT * KB * 2 / CG;           // B bytes per stage (per CTA)
+  static constexpr int NST = CG == 2 ? (DW_TMA ? 4 : (KIND == U_BWDG ? 5 : 6)) : STAGES;   // pipeline depth
+  static constexpr int A_ST = A_BYTES;                     // A bytes per stage
+  static constexpr int B_ST = BNT * BK * 2 / CG;           // B bytes per stage (per CTA)
   static constexpr int ST_B = A_ST + B_ST;
-  static constexpr int RES_B = RES ? 8 * A_BYTES : 0;      // resident A block (K <= 512)
-  static constexpr int CH_B = 64 * KB * 2;                 // one 64-wide MN-major chunk
-  static constexpr int PIPE_B = RES_B + NST * ST_B;
-  static constexpr int AUX_R = (RES || KIND == U_FWD) ? AUX_VEC       // forward: the per-tile vectors only
+  static constexpr int CH_B = 64 * BK * 2;                 // one 64-wide MN-major chunk
+  static constexpr int PIPE_B = NST * ST_B;
+  static constexpr int AUX_R = KIND == U_FWD ? AUX_VEC                // forward: the per-tile vectors only
                                : (KIND == U_DW ? 2 * NWB * WB_BUF + (DW_TMA ? 4 * DSTG : 0)
                                                : (NSB == 2 ? AUX_VEC + 2 * AUX_STG + (EPIW == 16 ? 2048 : 0) : AUX_REGION));
   static constexpr int SMEM = PIPE_B + AUX_BARS + AUX_R + 1024;
@@ -160,31 +137,25 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
   constexpr int HC = BN / NQ;             // accumulator columns per column group
   constexpr int EPI_THREADS = 32 * EPIW;
   static_assert(BNT == 256 || BNT == 128, "tile width");
-  static_assert(BNT == 256 || (KIND != U_FWDR && KIND != U_BWDG1), "narrow tiles: main kinds only");
   pdl_trigger();      // the next kernel's CTAs may take over SMs as this grid's tail drains
   // CTA pair: rank within the cluster, work is distributed over PAIRS
   const int crank = CG == 2 ? (int)ptx::cluster_ctarank() : 0;
   const int pair_id = (int)blockIdx.x / CG;
   const int npairs = (int)gridDim.x / CG;
-  constexpr bool IS_FWD = (KIND == U_FWD || KIND == U_FWDR);
-  constexpr bool RES = G_::RES;
-  constexpr int KB = G_::KB, NST = G_::NST, A_ST = G_::A_ST, ST_B = G_::ST_B;
-  constexpr int RES_B = G_::RES_B, CH_B = G_::CH_B, PIPE_B = G_::PIPE_B;
+  constexpr int NST = G_::NST, A_ST = G_::A_ST, ST_B = G_::ST_B, CH_B = G_::CH_B, PIPE_B = G_::PIPE_B;
   constexpr bool IS_DW = (KIND == U_DW || KIND == U_DWOPT || KIND == U_DWF);
-  constexpr bool IS_BWDG = (KIND == U_BWDG || KIND == U_BWDG1);
-  constexpr bool A_MN = (IS_BWDG || KIND == U_DX);
-  constexpr bool B_MN = (IS_FWD || IS_DW);
-  constexpr bool N_FAST = (IS_BWDG || IS_DW);   // tile order: n index fastest
+  constexpr bool A_MN = (KIND == U_BWDG || KIND == U_DX);
+  constexpr bool B_MN = (KIND == U_FWD || IS_DW);
+  constexpr bool N_FAST = (KIND == U_BWDG || IS_DW);   // tile order: n index fastest
   extern __shared__ uint8_t smem_raw[];
   // align to 1024 B (SWIZZLE_128B atoms) by adding an integer offset, so that the compiler
   // keeps the shared address space (ld.shared, not generic loads) for everything below
   uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint8_t* pipe = smem + RES_B;                                       // stage ring
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + PIPE_B);        // [8] (NST used)
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + PIPE_B);        // [8] (NST used), behind the stage ring smem[0, PIPE_B)
   uint64_t* empty = full + 8;                                         // [8]
   uint64_t* tfull = empty + 8;                                        // [2]
   uint64_t* tempty = tfull + 2;                                       // [2]
-  uint64_t* wfull = tempty + 2;                                       // DW: [half][buf]; FWDR: [0] = X resident
+  uint64_t* wfull = tempty + 2;                                       // DW: [half][buf]
   uint64_t* wempty = wfull + 8;                                       // DW: [half][buf]
   uint64_t* sfull = wempty + 8;                                       // DW (pairs): [half][2] staging buffer filled
   uint64_t* sempty = sfull + 4;                                       // DW (pairs): [half][2] ... drained by its TMA store
@@ -203,9 +174,9 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
   if (warp == 0 && ptx::elect_one()) {
     ptx::prefetch_tmap(&mapA);
     ptx::prefetch_tmap(&mapB);
-    if (IS_BWDG || KIND == U_DW || KIND == U_DX) ptx::prefetch_tmap(&mapC);
+    if (KIND == U_BWDG || KIND == U_DW || KIND == U_DX) ptx::prefetch_tmap(&mapC);
     if (G_::DW_TMA) { ptx::prefetch_tmap(&mapD); ptx::prefetch_tmap(&mapE); }
-    if (IS_BWDG) ptx::prefetch_tmap(&mapD);
+    if (KIND == U_BWDG) ptx::prefetch_tmap(&mapD);
   }
   if (warp == 1 && ptx::elect_one()) {
     for (int i = 0; i < NST; ++i) {
@@ -268,21 +239,6 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
     // ------------------------------------------------------------ TMA producer
     if (ptx::elect_one()) {
       uint32_t it = 0;
-      if (RES && pair_id < total) {
-        // the CTA's 128 batch rows of Xb, all of K, loaded once (grid % mt == 0)
-        const int nblk = (s.D + 63) / 64;
-        const int mrow = ((pair_id % g.mt) * CG + crank) * BM;
-        if (CG == 2) {
-          // both CTAs' blocks are counted on the leader's barrier (the leader issues the MMAs)
-          if (crank == 0) ptx::mbar_expect_tx(&wfull[0], 2 * nblk * A_BYTES);
-          for (int i = 0; i < nblk; ++i)
-            ptx::tma_load_2d_cg2(smem + i * A_BYTES, &mapA, &wfull[0], i * 64, mrow);
-        } else {
-          ptx::mbar_expect_tx(&wfull[0], nblk * A_BYTES);
-          for (int i = 0; i < nblk; ++i)
-            ptx::tma_load_2d(smem + i * A_BYTES, &mapA, &wfull[0], i * 64, mrow);
-        }
-      }
       for (int u = pair_id; u < total; u += npairs) {
         int z, m_idx, n_idx;
         decode(u, z, m_idx, n_idx);
@@ -293,14 +249,14 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
           const int st = it % NST;
           const uint32_t ph = (it / NST) & 1;
           ptx::mbar_wait(&empty[st], ph ^ 1);
-          uint8_t* sA = pipe + st * ST_B;
+          uint8_t* sA = smem + st * ST_B;
           uint8_t* sB = sA + A_ST;
-          int k0 = kb * KB, oa = 0, ob = 0;
+          int k0 = kb * BK, oa = 0, ob = 0;
           if (g.nseg > 1) {
             // x3: plane-pair segment of this K block; the plane offset goes to the INNER
             // coordinate of each operand's tensor (K for K-major loads, M/N for MN-major)
             const int seg = kb / g.kb_seg;
-            k0 = (kb - seg * g.kb_seg) * KB;
+            k0 = (kb - seg * g.kb_seg) * BK;
             oa = g.segA[seg];
             ob = g.segB[seg];
           }
@@ -315,12 +271,10 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
             // both CTAs load their A rows and their half of B; all bytes are counted on the
             // leader's full barrier, which only the leader arms
             if (crank == 0) ptx::mbar_expect_tx(&full[st], 2 * ST_B);
-            if (RES) {
-              // A is resident
-            } else if (A_MN) {
+            if (A_MN) {
 #pragma unroll
               for (int c = 0; c < BM / 64; ++c) {
-                if (IS_BWDG) ptx::tma_load_2d_cg2(sA + c * CH_B, &mapA, &full[st], 0, wb_row(m0 + c * 64, k0, oa));
+                if (KIND == U_BWDG) ptx::tma_load_2d_cg2(sA + c * CH_B, &mapA, &full[st], 0, wb_row(m0 + c * 64, k0, oa));
                 else ptx::tma_load_2d_cg2(sA + c * CH_B, &mapA, &full[st], mA + c * 64, kA);
               }
             } else {
@@ -329,7 +283,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
             if (B_MN) {
 #pragma unroll
               for (int c = 0; c < BN / 128; ++c) {
-                if (IS_FWD) ptx::tma_load_2d_cg2(sB + c * CH_B, &mapB, &full[st], 0,
+                if (KIND == U_FWD) ptx::tma_load_2d_cg2(sB + c * CH_B, &mapB, &full[st], 0,
                                                  wb_row(n0 + (crank * (BN / 128) + c) * 64, k0, ob));
                 else ptx::tma_load_2d_cg2(sB + c * CH_B, &mapB, &full[st], nB + (crank * (BN / 128) + c) * 64, kB);
               }
@@ -341,12 +295,10 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
             continue;
           }
           ptx::mbar_expect_tx(&full[st], ST_B);
-          if (RES) {
-            // A is resident
-          } else if (A_MN) {
+          if (A_MN) {
 #pragma unroll
             for (int c = 0; c < BM / 64; ++c) {
-              if (IS_BWDG) ptx::tma_load_2d(sA + c * CH_B, &mapA, &full[st], 0, wb_row(m0 + c * 64, k0, oa));
+              if (KIND == U_BWDG) ptx::tma_load_2d(sA + c * CH_B, &mapA, &full[st], 0, wb_row(m0 + c * 64, k0, oa));
               else ptx::tma_load_2d(sA + c * CH_B, &mapA, &full[st], mA + c * 64, kA);
             }
           } else {
@@ -355,7 +307,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
           if (B_MN) {
 #pragma unroll
             for (int c = 0; c < BN / 64; ++c) {
-              if (IS_FWD) ptx::tma_load_2d(sB + c * CH_B, &mapB, &full[st], 0, wb_row(n0 + c * 64, k0, ob));
+              if (KIND == U_FWD) ptx::tma_load_2d(sB + c * CH_B, &mapB, &full[st], 0, wb_row(n0 + c * 64, k0, ob));
               else ptx::tma_load_2d(sB + c * CH_B, &mapB, &full[st], nB + c * 64, kB);
             }
           } else if (KIND == U_DX) {
@@ -375,7 +327,6 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
       const uint32_t stepA = A_MN ? g.kstep_mn : 32u;
       const uint32_t stepB = B_MN ? g.kstep_mn : 32u;
       uint32_t it = 0, lt = 0;
-      if (RES && pair_id < total) ptx::mbar_wait(&wfull[0], 0);   // resident Xb landed
 #ifdef ASM_TIMING
       long long t_tempty = 0, t_full = 0, t_all = clock64();
 #endif
@@ -393,7 +344,6 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
         ptx::tc_fence_after();
         const uint32_t d_tmem = tmem_base + a * BN_FULL;
         for (int ki = 0; ki < nk; ++ki, ++it) {
-          const int kb = RES ? kblock(z, ki) : 0;     // only the resident-A variant addresses by kb
           const int st = it % NST;
           const uint32_t ph = (it / NST) & 1;
 #ifdef ASM_TIMING
@@ -404,12 +354,10 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
           t_full += clock64() - t1;
 #endif
           ptx::tc_fence_after();
-          // resident A: 64-wide K blocks of 16 KB; stage kb covers K = [32 kb, 32 kb + 32)
-          const uint32_t aA = RES ? ptx::smem_u32(smem + ((kb * KB) >> 6) * A_BYTES) + ((kb * KB) & 63) * 2u
-                                  : ptx::smem_u32(pipe + st * ST_B);
-          const uint32_t aB = ptx::smem_u32(pipe + st * ST_B) + A_ST;
+          const uint32_t aA = ptx::smem_u32(smem + st * ST_B);
+          const uint32_t aB = aA + A_ST;
 #pragma unroll
-          for (int kk = 0; kk < KB / 16; ++kk) {
+          for (int kk = 0; kk < BK / 16; ++kk) {
             if (CG == 2)
               ptx::umma_bf16_cg2(d_tmem, ptx::smem_desc(hiA, aA + kk * stepA),
                                  ptx::smem_desc(hiB, aB + kk * stepB), idesc,
@@ -437,7 +385,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
     // warps' hands: it waits for a staging buffer to be full, issues its two TMA stores (even /
     // odd d rows), waits until they have READ the buffer and hands it back.  The epilogue
     // warps never wait for a store, only -- two chunks later -- for the buffer.
-    if (G_::DW_TMA && g.dw_tma && lane < 2 && !ASM_DBG(g.debug_flags, 1)) {
+    if (G_::DW_TMA && g.dw_tma && lane < 2) {
       const int half = lane;
       const int dw_sh = g.dw_shift;
       // nothing reads dW inside the step: mark its lines evict-first so that they do not push
@@ -475,7 +423,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
     // Streams the bf16 weight block of each tile ([256 d x 128 classes], needed by the
     // normalisation-Jacobian correction in the epilogue) through a 2-deep ring per column
     // half, so the epilogue never waits on a global load.
-    if (KIND == U_DW && !ASM_DBG(g.debug_flags, 1) && ptx::elect_one()) {
+    if (KIND == U_DW && ptx::elect_one()) {
       uint32_t cc = 0;
       for (int u = pair_id; u < total; u += npairs) {
         int z, m_idx, n_idx;
@@ -536,8 +484,8 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
       int pz, pm, pn;
       decode(pu, pz, pm, pn);
       pm = pm * CG + crank;
-      if (IS_FWD) pre0 = s.inv_c[pn * BN + (et & (BN - 1))];
-      if (IS_BWDG) {
+      if (KIND == U_FWD) pre0 = s.inv_c[pn * BN + (et & (BN - 1))];
+      if (KIND == U_BWDG) {
         const int i = pn * BN + (et & (BN - 1));
         const bool iv = i < s.B;
         pre0 = iv ? s.negoff[i] : -INFINITY;                  // -(lse_i log2e) + log2(1/B)
@@ -595,12 +543,6 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
       float* v1 = vec1 + a * BN_FULL;
       float* v2 = vec2 + a * BN_FULL;
       uint32_t r0[32], r1[32];
-      if (ASM_DBG(g.debug_flags, 1)) {        // bring-up knob: mainloop only, no epilogue math
-        ptx::mbar_wait(&tfull[a], aph);
-        ptx::tc_fence_after();
-        release_acc(a);
-        continue;
-      }
 
       // The four 32-column chunks of this thread's half are read with the TMEM load of
       // chunk c+1 in flight while chunk c is processed; the accumulator stage is released
@@ -633,7 +575,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
       }                                                    \
       }
 
-      if (IS_FWD) {
+      if (KIND == U_FWD) {
         // ---- thread = batch row, columns = classes.  Stage 1/c_j for the tile in smem.
         if (et < BN) v0[et] = pre0;
         prefetch_tile(u + npairs);
@@ -702,7 +644,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
           }
         };
         ASM_EPILOGUE_CHUNKS(process)
-      } else if (IS_BWDG) {
+      } else if (KIND == U_BWDG) {
         // ---- thread = class j (row m), columns = batch rows i.  Stage the per-row terms.
         if (et < BN) {
           v0[et] = pre0;
@@ -972,7 +914,6 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
         // 128-byte line) before working on the current one: the loads that follow hit L2.
         const int ht = et & 127;
         auto prefetch_chunk = [&](int pm0, int pdb) {
-          if (ASM_DBG(g.debug_flags, 16)) return;              // A/B knob: no prefetch
           // [32 d x 128 classes] fp32 per array: 4 lines per row (+1 when the row is not
           // line-aligned, covered by the first 32 threads)
           const int row = ht >> 2;
@@ -1070,7 +1011,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
       }
 #undef ASM_EPILOGUE_CHUNKS
     }
-    if (IS_BWDG && EPIW == 16 && lt > 0) {
+    if (KIND == U_BWDG && EPIW == 16 && lt > 0) {
       named_bar_sync(1, EPI_THREADS);                        // the last tile's neighbour partials are in place
       if (q_prev_idx >= 0 && (half & 1) == 0)
         s.q_part[q_prev_idx] = q_prev + qx[(q_prev_a * 2 + (half >> 1)) * 128 + lane_row];
@@ -1080,11 +1021,11 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
       printf("TIMING kind %d pair %d warp %d: epilogue total %lld cyc, wait tfull %lld\n", KIND, pair_id, warp,
              clock64() - e_all, e_wait);
 #endif
-    if (IS_FWD && fwd_row >= 0)
+    if (KIND == U_FWD && fwd_row >= 0)
       s.part[(size_t)fwd_row * s.NT + (pair_id / g.mt) * NQ + half] = make_float2(run_m, run_z);
   }
 
-  if ((IS_BWDG || KIND == U_DX) && warp >= 4 && lane == 0) ptx::bulk_wait0();
+  if ((KIND == U_BWDG || KIND == U_DX) && warp >= 4 && lane == 0) ptx::bulk_wait0();
   ptx::tc_fence_before();
   __syncthreads();
   if (CG == 2) ptx::cluster_sync_all();       // the peer may still be read / signalled by the leader
@@ -1214,7 +1155,6 @@ bool umma_build_maps(UmmaMaps* m, const Step& s) {
   // the bf16 weights, column-blocked [planes * Cp/64 * D rows][64 classes]: every box is contiguous
   const uint64_t wrows = (uint64_t)(s.x3 ? 3 : 1) * (s.Cp / 64) * s.D;
   ok &= encode_map(&m->wb_mn, s.Wb, 64, wrows, 64, 64, 64);     // B of FWD / A of BWDG (MN-major)
-  ok &= encode_map(&m->wb_mn32, s.Wb, 64, wrows, 64, 64, 32);   // B of FWDR (32-deep K stages)
   ok &= encode_map(&m->wb_k, s.Wb, 64, wrows, 64, 64, 256);     // B of DX   (K-major, N = d)
   ok &= encode_map(&m->wb_k128, s.Wb, 64, wrows, 64, 64, 128);  // B half of DX in a CTA pair
   ok &= encode_map(&m->g_k, s.G, gi, s.Cp, gp, 64, 128);      // A of DW   (K-major: K = batch, M = class)
@@ -1279,12 +1219,11 @@ static const int kSegLo[6] = {0, 1, 0, 1, 2, 0};
 static const int kSegG[5] = {0, 0, 1, 1, 0};       // two-plane G'' against a three-plane operand
 static const int kSegO[5] = {0, 1, 0, 1, 2};
 
-static UmmaArgs base_args(const UmmaTuning& tu) {
+static UmmaArgs base_args() {
   UmmaArgs g{};
   g.desc_hi_k = ptx::make_smem_desc_hi(16, 1024);
-  g.desc_hi_mn = ptx::make_smem_desc_hi(tu.mn_lbo, tu.mn_sbo);
-  g.kstep_mn = tu.mn_kstep;
-  g.debug_flags = tu.debug_flags;
+  g.desc_hi_mn = ptx::make_smem_desc_hi(MN_LBO, MN_SBO);
+  g.kstep_mn = MN_KSTEP;
   g.ks = 1;
   return g;
 }
@@ -1312,11 +1251,6 @@ cudaError_t umma_configure() {
   cudaError_t e;
   if ((e = set_smem<U_FWD, 1>()) != cudaSuccess) return e;
   if ((e = set_smem<U_FWD, 2>()) != cudaSuccess) return e;
-#ifdef ASM_BRINGUP
-  if ((e = set_smem<U_FWDR, 1>()) != cudaSuccess) return e;
-  if ((e = set_smem<U_FWDR, 2>()) != cudaSuccess) return e;
-  if ((e = set_smem<U_BWDG1, 2>()) != cudaSuccess) return e;
-#endif
   if ((e = set_smem<U_BWDG, 1>()) != cudaSuccess) return e;
   if ((e = set_smem<U_BWDG, 2>()) != cudaSuccess) return e;
   if ((e = set_smem<U_DW, 1>()) != cudaSuccess) return e;
@@ -1337,7 +1271,7 @@ cudaError_t umma_configure() {
 
 void launch_umma_forward(const Step& s, const UmmaMaps& m, const UmmaTuning& tu, int num_sms,
                          cudaStream_t st) {
-  UmmaArgs g = base_args(tu);   // S = Xb Wb: lanes = batch rows, columns = classes
+  UmmaArgs g = base_args();   // S = Xb Wb: lanes = batch rows, columns = classes
   const int cg = fwd_cg(s.B, (tu.cg_mask & 1) ? 2 : 1);
   g.mt = ((s.B + BM - 1) / BM + cg - 1) / cg;
   const int bn = umma_tile_width(tu, cg, (long long)g.mt * (s.Cp / BN_FULL), num_sms);
@@ -1348,23 +1282,6 @@ void launch_umma_forward(const Step& s, const UmmaMaps& m, const UmmaTuning& tu,
     launch_k<U_FWD, 2, 128>(units, m.xb_k, m.wb_mn, m.wb_mn, s, g, st);
     return;
   }
-#ifdef ASM_BRINGUP
-  if (s.D <= 512 && (tu.debug_flags & 4) && cg == 2 && !s.x3) {
-    // opt-in: Xb row tiles resident in both CTAs of a pair, only the weight halves stream
-    g.kb_total = (s.D + BK - 1) / BK;
-    g.kb_per = g.kb_total;
-    launch_k<U_FWDR, 2>(units, m.xb_k, m.wb_mn, m.wb_mn, s, g, st);
-    return;
-  }
-  if (s.D <= 512 && (tu.debug_flags & 4) && cg == 1 && !s.x3) {   // opt-in: measured slower (55 vs 48 us)
-    // Xb row tile resident in shared memory, weights stream in 32-deep K stages
-    g.kb_total = (s.D + 31) / 32;
-    g.kb_per = g.kb_total;
-    g.desc_hi_mn = ptx::make_smem_desc_hi(Geo<U_FWDR>::CH_B, tu.mn_sbo);   // chunk stride 4 KB
-    launch_k<U_FWDR, 1>(units, m.xb_k, m.wb_mn32, m.wb_mn32, s, g, st);
-    return;
-  }
-#endif
   set_segments(g, s.x3 != 0, (s.D + BK - 1) / BK, kSegHi, kSegLo, x3_segments(), s.D, 1);
   if (cg == 2) launch_k<U_FWD, 2>(units, m.xb_k, m.wb_mn, m.wb_mn, s, g, st);
   else launch_k<U_FWD, 1>(units, m.xb_k, m.wb_mn, m.wb_mn, s, g, st);
@@ -1372,7 +1289,7 @@ void launch_umma_forward(const Step& s, const UmmaMaps& m, const UmmaTuning& tu,
 
 void launch_umma_bwdg(const Step& s, const UmmaMaps& m, const UmmaTuning& tu, int num_sms,
                       cudaStream_t st) {
-  UmmaArgs g = base_args(tu);   // recompute S^T -> G'' (bf16) + q_part: lanes = classes
+  UmmaArgs g = base_args();   // recompute S^T -> G'' (bf16) + q_part: lanes = classes
   const int cg = (tu.cg_mask & 2) ? 2 : 1;
   g.mt = s.Cp / (BM * cg);
   const int bn = umma_tile_width(tu, cg, (long long)g.mt * ((s.B + BN_FULL - 1) / BN_FULL), num_sms);
@@ -1382,16 +1299,13 @@ void launch_umma_bwdg(const Step& s, const UmmaMaps& m, const UmmaTuning& tu, in
   g.rev = tu.l2_order ? 1 : 0;  // the forward kernel swept the classes upwards: start where it stopped
   const int units = min(g.mt * g.nt, num_sms / cg);
   if (bn == 128) launch_k<U_BWDG, 2, 128>(units, m.wb_mn, m.xb_mn, m.g_st, s, g, st, &m.g_st32);   // X box: 64 rows per CTA
-#ifdef ASM_BRINGUP
-  else if (cg == 2 && (tu.debug_flags & 8)) launch_k<U_BWDG1, 2>(units, m.wb_mn, m.xb_k, m.g_st, s, g, st);
-#endif
   else if (cg == 2) launch_k<U_BWDG, 2>(units, m.wb_mn, m.xb_k, m.g_st, s, g, st, &m.g_st32);
   else launch_k<U_BWDG, 1>(units, m.wb_mn, m.xb_k256, m.g_st, s, g, st);
 }
 
 void launch_umma_dw(const Step& s, const UmmaMaps& m, const UmmaTuning& tu, int num_sms,
                     cudaStream_t st) {
-  UmmaArgs g = base_args(tu);   // dW^T = G''^T Xb - correction: lanes = classes, columns = d
+  UmmaArgs g = base_args();   // dW^T = G''^T Xb - correction: lanes = classes, columns = d
   const int cg = (tu.cg_mask & 4) ? 2 : 1;
   g.mt = s.Cp / (BM * cg);
   const int bn = umma_tile_width(tu, cg, (long long)g.mt * ((s.D + BN_FULL - 1) / BN_FULL), num_sms);
@@ -1425,7 +1339,7 @@ void launch_umma_dw(const Step& s, const UmmaMaps& m, const UmmaTuning& tu, int 
 
 void launch_umma_dx(const Step& s, const UmmaMaps& m, const UmmaTuning& tu, int num_sms,
                     cudaStream_t st) {
-  UmmaArgs g = base_args(tu);   // dX partials = G'' Wb^T, split over the classes
+  UmmaArgs g = base_args();   // dX partials = G'' Wb^T, split over the classes
   const int cg = fwd_cg(s.B, (tu.cg_mask & 8) ? 2 : 1);
   g.mt = ((s.B + BM - 1) / BM + cg - 1) / cg;
   g.nt = (s.D + BN - 1) / BN;
