@@ -8,6 +8,7 @@ B200 A-softmax head, driven like the reference's train loop (train.py:223-250).
         examples/train_sphereface20.py --batch 512        # DDP backbone + class-sharded head
     python examples/train_sphereface20.py --margin arcface --scale 64 --margin-value 0.5
     python examples/train_sphereface20.py --loss focal --focal-gamma 1 --focal-alpha 2
+    python examples/train_sphereface20.py --margin softmax     # the reference's plain x.w classifier
 
 Only the head is this repository's product; the backbone is ordinary PyTorch (the survey
 marks backbones out of scope) and exists to show where the head plugs in:
@@ -25,7 +26,8 @@ import torch
 import torch.nn as nn
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from tf_face_toolbox_b200 import AdditiveMargin, FocalLoss, FusedOptimizer, LambdaState, asoftmax_head  # noqa: E402
+from tf_face_toolbox_b200 import (AdditiveMargin, FocalLoss, FusedOptimizer, LambdaState, LinearSoftmax,  # noqa: E402
+                                  asoftmax_head)
 
 
 class ResBlock(nn.Module):
@@ -89,8 +91,9 @@ def main():
     ap.add_argument("--lr", type=float, default=0.01)
     ap.add_argument("--mode", default="bf16")
     ap.add_argument("--transport", default="nvlink", help="multi-GPU exchanges: nvlink | nccl")
-    ap.add_argument("--margin", default="asoftmax", choices=["asoftmax", "arcface", "cosface"],
-                    help="A-softmax (m = 4, annealed lambda), or an additive margin on normalised embeddings")
+    ap.add_argument("--margin", default="asoftmax", choices=["asoftmax", "arcface", "cosface", "softmax"],
+                    help="A-softmax (m = 4, annealed lambda), an additive margin on normalised embeddings, "
+                         "or the reference's plain softmax classifier (logits x.w, no margin)")
     ap.add_argument("--scale", type=float, default=64.0, help="s of the additive margins")
     ap.add_argument("--margin-value", type=float, default=None,
                     help="m2 of ArcFace (default 0.5) or m3 of CosFace (default 0.35)")
@@ -104,6 +107,8 @@ def main():
         margin = AdditiveMargin.arcface(args.scale, 0.5 if args.margin_value is None else args.margin_value)
     elif args.margin == "cosface":
         margin = AdditiveMargin.cosface(args.scale, 0.35 if args.margin_value is None else args.margin_value)
+    elif args.margin == "softmax":
+        margin = LinearSoftmax()
     else:
         margin = None
     # under torchrun: data-parallel backbone (DDP) + class-parallel head, one rank per GPU
@@ -158,7 +163,8 @@ def main():
         loss = head_step(net, images, labels, head_call, opt_backbone, world=world)
         losses.append(loss)
         if rank == 0 and (step % 5 == 0 or step == args.steps - 1):
-            extra = f"  lambda {lam.value():.2f}" if margin is None else f"  {args.margin} s={margin.s:g}"
+            extra = (f"  lambda {lam.value():.2f}" if margin is None
+                     else f"  {args.margin} s={margin.s:g}" if isinstance(margin, AdditiveMargin) else "  softmax")
             name = "focal_loss" if loss_kind is not None else "cross_entropy"
             print(f"step {step:4d}  {name} {float(loss):.4f}{extra}", flush=True)
     torch.cuda.synchronize()

@@ -237,10 +237,16 @@ int asm_set_embedding_dtype(asm_head* h, int32_t bytes_per_element);
  *                                         = t - m2 sin(m2) - m3          otherwise (no "easy margin").
  *                                  m2 = 0: CosFace (s (cos theta - m3)); m3 = 0: ArcFace
  *                                  (s cos(theta + m2)).  lambda and cfg.m are ignored.
- * margin == NULL restores the default.  s must be finite and > 0, m2 in [0, pi/2], m3 finite and
- * >= 0; anything else returns ASM_ERR_INVALID_ARG and changes nothing.
+ *   ASM_MARGIN_LINEAR              the plain bias-free classifier of the reference's networks
+ *                                  (nets/sphere.py:84-111): f_ij = x_i.w_j for every j, target
+ *                                  included, with no norms and no margin.  dX = g W^T, dW = X^T g with
+ *                                  g = (softmax(f) - onehot)/B.  s, m2, m3, lambda and cfg.m are ignored.
+ * margin == NULL restores the default.  For ASM_MARGIN_ADDITIVE s must be finite and > 0, m2 in
+ * [0, pi/2], m3 finite and >= 0; anything else, or a kind not listed here, returns ASM_ERR_INVALID_ARG
+ * and changes nothing.  Kind 2 is deliberately left unassigned: earlier releases rejected it, and
+ * callers that probe the argument check with it keep getting ASM_ERR_INVALID_ARG.
  */
-enum { ASM_MARGIN_ASOFTMAX = 0, ASM_MARGIN_ADDITIVE = 1 };
+enum { ASM_MARGIN_ASOFTMAX = 0, ASM_MARGIN_ADDITIVE = 1, ASM_MARGIN_LINEAR = 3 };
 typedef struct {
   int32_t kind;
   float   s, m2, m3;

@@ -49,7 +49,7 @@ class AsmMargin(C.Structure):
     _fields_ = [("kind", C.c_int32), ("s", C.c_float), ("m2", C.c_float), ("m3", C.c_float)]
 
 
-MARGIN_ASOFTMAX, MARGIN_ADDITIVE = 0, 1
+MARGIN_ASOFTMAX, MARGIN_ADDITIVE, MARGIN_LINEAR = 0, 1, 3
 
 
 class AsmLoss(C.Structure):

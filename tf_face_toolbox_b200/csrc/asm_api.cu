@@ -45,6 +45,7 @@ struct asm_head {
   P2P p2p{};
   bool p2p_ready = false;
   float* Xg = nullptr;           // [B_max, D] gathered embeddings
+  float* wzero = nullptr;        // [Cp] zeros (workspace): Step::wcorr of the linear kind
   int launches = 0;
   // optional per-kernel timing (asm_set_profiling): event i is recorded before kernel i
   bool profiling = false;
@@ -64,7 +65,7 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct Layout {
   size_t ylocal, flags, n, inv_n, inv_c, margin, tgt_s, tgt_f, part, stats_local, lse, negoff, gtarget, rcoef, rowloss, rowgrad, counter,
-      q_part, G, dx_part, Xb, Wb, Xs, Xg, step_dev, wsq_part, wsq_ticket, total;
+      q_part, G, dx_part, Xb, Wb, Xs, Xg, step_dev, wsq_part, wsq_ticket, wzero, total;
   int Cp, NT, MT;
   size_t dx_capacity;
 };
@@ -144,6 +145,7 @@ Layout make_layout(const asm_config& c, int num_sms) {
     L.step_dev = take(256);
   }
   L.rowgrad = take(B * 4);   // last: every buffer before it keeps the offset it had without it
+  L.wzero = take((size_t)L.Cp * 4);   // zeroed once, never written: the linear kind's dW correction scale
   L.total = off;
   return L;
 }
@@ -196,7 +198,7 @@ int dx_sms(const asm_head* h) { return split_active(h) ? h->num_sms - 2 * h->dw_
 // that operand is the scaled, normalised copy Xs the norm kernel wrote.
 Step simt_step(const Step& s) {
   Step t = s;
-  if (s.mg.kind != 0) t.X = s.Xs;
+  if (s.mg.kind == kMarginAdditive) t.X = s.Xs;
   return t;
 }
 
@@ -319,7 +321,7 @@ int run_backward(asm_head* h, const float* stats_all, int n_shards, float* loss_
       mark(h, "dx_gemm", sx, !h->phase_profiling);
       if (tc) launch_umma_dx(s, h->maps, h->tune, dx_sms(h), sx);
       else launch_simt_dx(simt_step(s), sx);
-      const bool add = s.mg.kind != 0;
+      const bool add = s.mg.kind == kMarginAdditive;
       mark(h, tp ? (add ? "dx_finish_margin_exchange" : "dx_finish_exchange") : (add ? "dx_finish_margin" : "dx_finish"), sx,
            !h->phase_profiling);
       if (tp) launch_dx_finish_p2p(s, *tp, sx);
@@ -458,6 +460,8 @@ int asm_create(asm_head** out, const asm_config* cfg) {
   s.rcoef = (float*)(w + L.rcoef);
   s.rowloss = (float*)(w + L.rowloss);
   s.rowgrad = (float*)(w + L.rowgrad);
+  h->wzero = (float*)(w + L.wzero);
+  s.wcorr = s.inv_c;
   s.counter = (unsigned int*)(w + L.counter);
   s.q_part = (float*)(w + L.q_part);
   s.wsq_part = (float*)(w + L.wsq_part);
@@ -710,7 +714,7 @@ int asm_set_margin(asm_head* h, const asm_margin* margin) {
     const float s = margin->s, m2 = margin->m2, m3 = margin->m3;
     if (!(isfinite(s) && s > 0.f) || !(m2 >= 0.f && m2 <= (float)(M_PI / 2)) || !(isfinite(m3) && m3 >= 0.f))
       return fail(h, ASM_ERR_INVALID_ARG, "additive margin needs finite s > 0, m2 in [0, pi/2], finite m3 >= 0%s", "");
-    g.kind = 1;
+    g.kind = kMarginAdditive;
     g.s = s;
     g.inv_s = (float)(1.0 / (double)s);
     g.cm = (float)cos((double)m2);
@@ -718,10 +722,14 @@ int asm_set_margin(asm_head* h, const asm_margin* margin) {
     g.tau = (float)cos(M_PI - (double)m2);
     g.fb = (float)((double)m2 * sin((double)m2) + (double)m3);
     g.m3 = m3;
+  } else if (margin && margin->kind == ASM_MARGIN_LINEAR) {
+    g.kind = kMarginLinear;                 // s, m2, m3 are ignored
   } else if (margin && margin->kind != ASM_MARGIN_ASOFTMAX) {
     return fail(h, ASM_ERR_INVALID_ARG, "unknown margin kind%s", "");
   }
   h->st.mg = g;
+  // the linear kind's dW has no normalisation term: its coefficient reads zeros instead of 1/c_j
+  h->st.wcorr = g.kind == kMarginLinear ? h->wzero : h->st.inv_c;
   return ASM_OK;
 }
 

@@ -45,10 +45,13 @@ __device__ __forceinline__ void psi_eval(float t, int m, float& psi, float& dpsi
 // GEMMs then see s * x_i / n_i, so a raw logit is s * cos(theta) and t = logit / s.
 //   t >= tau = cos(pi - m2):  phi = cos(theta + m2) - m3,  phi' = cos m2 + t sin m2 / sin(theta)
 //   otherwise:                phi = t - m2 sin m2 - m3,    phi' = 1
-// (the usual non-"easy-margin" fallback; phi jumps at tau).  kind == 0: A-softmax instead.
+// (the usual non-"easy-margin" fallback; phi jumps at tau).  kind == 0: A-softmax instead;
+// kind == 3: the plain linear classifier f_ij = x_i.w_j (DESIGN.md section 2.3), no margin at all.
 // ---------------------------------------------------------------------------------------
+constexpr int kMarginAdditive = 1;
+constexpr int kMarginLinear = 3;
 struct Margin {
-  int kind;                  // 0 = A-softmax (psi, lambda), 1 = additive (s, m2, m3)
+  int kind;                  // 0 = A-softmax (psi, lambda), 1 = additive (s, m2, m3), 3 = linear
   float s, inv_s;            // scale and 1/s
   float cm, sm;              // cos m2, sin m2
   float tau;                 // cos(pi - m2)

@@ -180,6 +180,9 @@ struct Step {
   // rcoef and rowgrad, so no GEMM kernel sees it.
   LossParams ls;
   float* rowgrad;            // [B]   invB * gscale * w_i: the CUDA-core recompute's per-row gradient factor
+  // [Cp] per-class scale of the normalisation term of dW: coef_j = -q_j wcorr_j^2 + wd_g.  inv_c for
+  // A-softmax and the additive margin; an all-zero array for the linear kind, whose dW has no such term.
+  const float* wcorr;
 };
 
 // prep: column norms of W (+ bf16 copy), row norms of X (+ bf16 copy), label localisation.

@@ -170,7 +170,7 @@ __global__ void __launch_bounds__(256) dx_finish_margin_p2p_kernel(Step s, P2P p
 }
 
 void launch_dx_finish_p2p(const Step& s, const P2P& p, cudaStream_t st) {
-  if (s.mg.kind != 0) {
+  if (s.mg.kind == kMarginAdditive) {
     int blocks = (s.B + 1) / 2;
     if (blocks > 148 * 2) blocks = 148 * 2;
     launch_pdl(dx_finish_margin_p2p_kernel, dim3(blocks), dim3(256), 0, st, s.pdl != 0, 1, s, p);

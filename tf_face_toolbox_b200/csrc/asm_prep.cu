@@ -211,7 +211,10 @@ __device__ __forceinline__ void prep_block(const Step& s, const void* labels, in
 #pragma unroll
       for (int r = 0; r < TY; ++r) acc += red[r][t];
       const int j = bid * 2 * TX + t;
-      if (j < s.Cp) s.inv_c[j] = (j < s.C && acc > 0.f) ? rsqrtf(acc) : 0.f;
+      // linear kind: f_ij = x_i.w_j, so 1/c_j := 1 (a zero column gives logit 0, not a masked class);
+      // the column sums are still needed for reg_loss
+      if (j < s.Cp)
+        s.inv_c[j] = s.mg.kind == kMarginLinear ? (j < s.C ? 1.0f : 0.f) : ((j < s.C && acc > 0.f) ? rsqrtf(acc) : 0.f);
       if (s.reg_out) red[0][t] = j < s.C ? acc : 0.f;
     }
     if (s.reg_out) {
@@ -353,7 +356,7 @@ static void launch_prep_t(const Step& s, const void* labels, int label_bytes, cu
 
 template <int TX, int TY, int U>
 static void launch_prep_t(const Step& s, const void* labels, int label_bytes, cudaStream_t st, const P2P* p) {
-  if (s.mg.kind != 0) launch_prep_t<TX, TY, U, true>(s, labels, label_bytes, st, p);
+  if (s.mg.kind == kMarginAdditive) launch_prep_t<TX, TY, U, true>(s, labels, label_bytes, st, p);
   else launch_prep_t<TX, TY, U, false>(s, labels, label_bytes, st, p);
 }
 
@@ -505,7 +508,7 @@ __global__ void __launch_bounds__(256) dx_finish_margin_kernel(Step s) {
 }
 
 void launch_dx_finish(const Step& s, cudaStream_t st) {
-  if (s.mg.kind != 0) {
+  if (s.mg.kind == kMarginAdditive) {
     int blocks = (s.B + 1) / 2;
     if (blocks > 148 * 8) blocks = 148 * 8;
     launch_pdl(dx_finish_margin_kernel, dim3(blocks), dim3(256), 0, st, s.pdl != 0, 1, s);

@@ -12,7 +12,7 @@ namespace asmh {
 //   g_y = (e^{f_y - lse} - 1)/B,  G'_y = g_y (lambda + psi')/(1 + lambda),
 //   r   = g_y (psi - t psi') / ((1 + lambda) n)            (SURVEY.md 8a, row a3)
 // or, for the additive margin, G'_y = g_y phi'(t) with t = s_y / s, and r = 0 (the projection of
-// dx_finish_rows_margin replaces the r_i x_i term).
+// dx_finish_rows_margin replaces the r_i x_i term); for the linear kind G'_y = g_y and r = 0.
 // A row whose label lies outside [0, C_total) (ylocal == -2) has no defined loss: it gets NaN,
 // as the reference's sparse_softmax_cross_entropy does on the GPU (nets/sphere.py:109).
 //
@@ -51,10 +51,12 @@ __device__ __forceinline__ void row_epilogue(const Step& s, int row, float m, fl
   s.rowgrad[row] = focal ? gB * w : gB;
   s.rowloss[row] = yl_row == -2 ? __int_as_float(0x7fc00000) : loss;
   float gt = 0.f, r = 0.f;
-  if (owned && s.mg.kind != 0) {                 // additive: G'_y = g_y phi'(t), r = 0
+  if (owned && s.mg.kind == kMarginAdditive) {   // additive: G'_y = g_y phi'(t), r = 0
     float phi, dphi;
     phi_eval(tgt_s_row * s.mg.inv_s, s.mg, phi, dphi);
     gt = (expf(tgt_f_row - lse) - 1.0f) * gB * dphi;
+  } else if (owned && s.mg.kind == kMarginLinear) {   // linear: G'_y = g_y, r = 0
+    gt = (expf(tgt_f_row - lse) - 1.0f) * gB;
   } else if (owned) {
     float psi, dpsi;
     const float t = fminf(1.f, fmaxf(-1.f, tgt_s_row * inv_n_row));

@@ -166,8 +166,9 @@ __global__ void __launch_bounds__(256) simt_kernel(Step s, int k_per_split) {
         float v = acc[a][b] * ic[b];
         if (rv && j == yl) {
           s.tgt_s[i] = v;
-          v = s.mg.kind != 0 ? additive_logit(v, s.mg)
-                             : target_logit(v, s.n[i], s.inv_n[i], s.m, step_lambda(s.lambda, s.lambda_dev));
+          if (s.mg.kind == kMarginAdditive) v = additive_logit(v, s.mg);
+          else if (s.mg.kind != kMarginLinear)
+            v = target_logit(v, s.n[i], s.inv_n[i], s.m, step_lambda(s.lambda, s.lambda_dev));
           s.tgt_f[i] = v;
         }
         if (j >= s.C) v = -INFINITY;
@@ -241,7 +242,7 @@ __global__ void __launch_bounds__(256) simt_kernel(Step s, int k_per_split) {
       if (j >= s.C) continue;
       float q = 0.f;
       for (int t = 0; t < s.MT; ++t) q += s.q_part[(size_t)t * s.Cp + j];
-      const float ic = s.inv_c[j];
+      const float ic = s.wcorr[j];
       const float coef = q * ic * ic;
 #pragma unroll
       for (int a = 0; a < 8; ++a) {

@@ -119,7 +119,9 @@ __device__ __noinline__ float fwd_target(float* tgt_s, float* tgt_f, const float
                                          float sv) {
   tgt_s[row] = sv;
   const Margin mg = *margin_record(tgt_s);
-  const float fv = mg.kind != 0 ? additive_logit(sv, mg) : target_logit(sv, n[row], inv_n[row], m, lambda);
+  const float fv = mg.kind == kMarginAdditive ? additive_logit(sv, mg)
+                   : mg.kind == kMarginLinear ? sv
+                                              : target_logit(sv, n[row], inv_n[row], m, lambda);
   tgt_f[row] = fv;
   return fv;
 }
@@ -499,7 +501,7 @@ umma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CU
         const float* qp = s.q_part + pj;
         pre0 = qp[0];
         pre1 = s.MT > 1 ? qp[(size_t)s.Cp] : 0.f;
-        pre2 = s.inv_c[pj];
+        pre2 = s.wcorr[pj];
         pre3 = s.MT > 2 ? qp[(size_t)2 * s.Cp] : 0.f;
         pre4 = s.MT > 3 ? qp[(size_t)3 * s.Cp] : 0.f;
         pre5 = 0.f;

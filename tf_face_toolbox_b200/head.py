@@ -86,6 +86,25 @@ class AdditiveMargin:
 
 
 # --------------------------------------------------------------------------------------
+# the reference's plain classifier: bias-free fully_connected + softmax cross-entropy
+# --------------------------------------------------------------------------------------
+@dataclass(frozen=True)
+class LinearSoftmax:
+    """Unnormalised logits f_ij = x_i . w_j for every class, target included: no norms, no margin.
+    This is the `fully_connected(features, num_classes)` (no bias) + sparse_softmax_cross_entropy
+    slot of every network in the reference (nets/sphere.py:84-111, nets/resnet.py:151-177,
+    nets/shufflenet_v2.py:179-208).  Pass it as `margin=` to the head's entry points; `m` and
+    lambda are then ignored.  Weight decay, grad_scale, the fused optimizer and `loss=` compose
+    as they do for the other heads."""
+
+    def _struct(self) -> "_lib.AsmMargin":
+        return _lib.AsmMargin(_lib.MARGIN_LINEAR, 0.0, 0.0, 0.0)
+
+
+Margin = (AdditiveMargin, LinearSoftmax)
+
+
+# --------------------------------------------------------------------------------------
 # focal loss (loss.py:18-27 of the reference) in place of the softmax cross-entropy
 # --------------------------------------------------------------------------------------
 @dataclass(frozen=True)
@@ -118,7 +137,7 @@ def _as_lambda(lambda_state) -> float:
 class _Handle:
     def __init__(self, device: torch.device, D: int, C_total: int, C_local: int, class_offset: int,
                  B_max: int, m: int, mode: str, rank: int = 0, world: int = 1,
-                 margin: Optional[AdditiveMargin] = None, loss: Optional[FocalLoss] = None):
+                 margin=None, loss: Optional[FocalLoss] = None):
         self.lib = _lib.load()
         if device.type != "cuda":
             raise RuntimeError("the A-softmax head runs on a CUDA (B200) device only; no CPU fallback")
@@ -170,14 +189,14 @@ def _round_batch(B: int) -> int:
 
 
 def get_handle(device, D, C_total, C_local, class_offset, B, m, mode, rank=0, world=1, tag=None,
-               margin: Optional[AdditiveMargin] = None, loss: Optional[FocalLoss] = None) -> _Handle:
+               margin=None, loss: Optional[FocalLoss] = None) -> _Handle:
     """`tag` separates handles with different per-handle state (e.g. a CUDA-graph step that
     reads lambda from device memory) from the plain eager ones."""
     device = torch.device(device)
     if device.index is None:
         device = torch.device("cuda", torch.cuda.current_device())
-    if margin is not None and not isinstance(margin, AdditiveMargin):
-        raise TypeError("margin must be None (A-softmax) or an AdditiveMargin")
+    if margin is not None and not isinstance(margin, Margin):
+        raise TypeError("margin must be None (A-softmax), an AdditiveMargin or LinearSoftmax()")
     if loss is not None and not isinstance(loss, FocalLoss):
         raise TypeError("loss must be None (softmax cross-entropy) or a FocalLoss")
     key = (device.index, D, C_total, C_local, class_offset, _round_batch(B), m, mode, rank, world, margin, loss, tag)
@@ -267,7 +286,7 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
                   return_logits: bool = False, compute_grads: bool = True,
                   check_labels: bool = False, optimizer: Optional["FusedOptimizer"] = None,
                   grad_scale: float = 1.0, weight_decay: float = 0.0,
-                  reg_loss_out: Optional[torch.Tensor] = None, margin: Optional[AdditiveMargin] = None,
+                  reg_loss_out: Optional[torch.Tensor] = None, margin=None,
                   loss: Optional[FocalLoss] = None, _handle_tag=None
                   ) -> Tuple[torch.Tensor, Optional[torch.Tensor], Optional[torch.Tensor], Optional[torch.Tensor]]:
     """A-softmax head forward + backward on one GPU that owns every class.
@@ -288,6 +307,8 @@ def asoftmax_head(embeddings: torch.Tensor, labels: torch.Tensor, num_classes: i
     without reg_loss.
     `margin` (an AdditiveMargin) selects the ArcFace / CosFace head on normalised embeddings
     instead of A-softmax; `m` and lambda_state are then ignored.  None: A-softmax.
+    `margin=LinearSoftmax()` is the reference's plain classifier: logits x_i . w_j, no margin,
+    `m` and lambda_state ignored.
     `loss` (a FocalLoss) replaces the softmax cross-entropy by the reference's focal loss on the
     same logits; loss, dX and dW are then those of the focal loss.  None: cross-entropy.
     Asynchronous on the current CUDA stream.
@@ -367,7 +388,7 @@ class GraphedASoftmaxStep:
     """
 
     def __init__(self, weights: torch.Tensor, batch_size: int, m: int = 4, mode: str = "bf16",
-                 labels_dtype=torch.int32, margin: Optional[AdditiveMargin] = None,
+                 labels_dtype=torch.int32, margin=None,
                  loss: Optional[FocalLoss] = None):
         assert weights.is_cuda and weights.dtype == torch.float32 and weights.is_contiguous()
         dev = weights.device
@@ -432,7 +453,7 @@ class ASoftmaxLoss(torch.autograd.Function):
     gradient the caller promises to send into this loss (1.0 for a plain `loss.backward()`, the loss
     scale otherwise): it is applied inside the kernels and backward returns the stored gradients
     untouched -- no pass over [D, C].  Without it backward multiplies by the incoming gradient.
-    `margin` (an AdditiveMargin, or None for A-softmax) and `loss` (a FocalLoss, or None for the
+    `margin` (an AdditiveMargin, LinearSoftmax(), or None for A-softmax) and `loss` (a FocalLoss, or None for the
     cross-entropy) as in asoftmax_head."""
 
     @staticmethod
@@ -464,13 +485,18 @@ class ASoftmaxHead:
 
     `features` are the backbone's embeddings (the reference passes images to the full
     network; the head is the part after `features = self.backbone(images)`, nets/sphere.py:82).
+
+    With `margin=LinearSoftmax()` the head also takes the order in which `Singular` and
+    `DataParallel` drive a plain classifier (data_parallel.py:51, :133): forward without labels
+    returns {'logits': None, 'features': features}, and loss_function(scope, labels, **logits)
+    runs the fused step.
     """
     name = "classifier"
 
     def __init__(self, num_features: int, num_classes: int, m: int = 4, weight_decay: float = 5e-4,
                  mode: str = "bf16", device="cuda", lambda_state: Optional[LambdaState] = None,
                  return_logits: bool = False, seed: Optional[int] = None, num_gpus: int = 1,
-                 mult_lr: float = 1.0, margin: Optional[AdditiveMargin] = None,
+                 mult_lr: float = 1.0, margin=None,
                  loss: Optional[FocalLoss] = None):
         gen = None
         if seed is not None:
@@ -480,7 +506,8 @@ class ASoftmaxHead:
         self.weights = w.to(device)                  # classifier/fc_classifier/weights [D, C]
         self.num_classes = num_classes
         self.m = m
-        self.margin = margin                         # None: A-softmax; AdditiveMargin: ArcFace / CosFace
+        self.margin = margin                         # None: A-softmax; AdditiveMargin: ArcFace / CosFace;
+                                                     # LinearSoftmax: the plain classifier
         self.loss = loss                             # None: cross-entropy; FocalLoss: loss.py's focal_loss
         self.weight_decay = weight_decay
         self.mode = mode
@@ -491,13 +518,23 @@ class ASoftmaxHead:
         self.num_gpus, self.mult_lr = num_gpus, mult_lr
         self._reg = torch.zeros(1, device=self.weights.device, dtype=torch.float32)
         self._last = None
+        self._pending = None                         # num_classes of a forward without labels (LinearSoftmax)
 
     # nets/net_base.py:84-86, margin form data_parallel.py:220
     def forward(self, features, labels=None, num_classes=None, is_training=True):
         if not is_training:
             return features                           # nets/sphere.py:96-101: bare features
         assert num_classes is not None, "num_classes must be given when is_training=True"
+        if labels is None and isinstance(self.margin, LinearSoftmax):
+            # non-margin tower order: the labels arrive with loss_function, which runs the step
+            self._last = None
+            self._pending = num_classes
+            return {"logits": None, "features": features}
         assert labels is not None, "a margin head needs labels in forward (data_parallel.py:220)"
+        self._run(features, labels, num_classes)
+        return {"logits": self._last["logits"], "features": features}
+
+    def _run(self, features, labels, num_classes):
         lam = self.lambda_state.step()                # global_step += 1, first step uses it = 1
         scale = self.mult_lr / self.num_gpus
         loss, logits, dX, dW = asoftmax_head(features, labels, num_classes, self.m, lam,
@@ -505,12 +542,16 @@ class ASoftmaxHead:
                                              return_logits=self.return_logits, grad_scale=scale,
                                              weight_decay=self.weight_decay, reg_loss_out=self._reg,
                                              margin=self.margin, loss=self.loss)
-        self._last = dict(loss=loss, dX=dX, dW=dW, lam=lam, scale=scale, reg=self._reg[0].clone())
-        out = {"logits": logits, "features": features}
-        return out
+        self._last = dict(loss=loss, dX=dX, dW=dW, lam=lam, scale=scale, reg=self._reg[0].clone(),
+                          logits=logits)
+        self._pending = None
 
     # nets/net_base.py:88-90; nets/sphere.py:103-118
     def loss_function(self, scope, labels, **logits):
+        if self._last is None and self._pending is not None:
+            # forward(features, num_classes=C) of the non-margin order left the step to this call
+            self._run(logits["features"], labels, self._pending)
+            self._pending = None
         assert self._last is not None, "forward(...) must run first"
         losses = [self._last["loss"]]
         losses_name = ["focal_loss" if self.loss is not None else "cross_entropy"]
@@ -519,7 +560,7 @@ class ASoftmaxHead:
         losses.append(self._last["reg"])
         losses_name.append("reg_loss")
         others = OrderedDict()
-        if self.margin is None:                       # lambda means nothing to the additive margins
+        if self.margin is None:                       # lambda means nothing to the other kinds
             others["lambda"] = self._last["lam"]
         return losses, losses_name, others
 

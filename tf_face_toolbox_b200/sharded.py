@@ -24,7 +24,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from .head import AdditiveMargin, FocalLoss, LambdaState, _as_lambda, get_handle
+from .head import FocalLoss, LambdaState, _as_lambda, get_handle
 
 
 def shard_bounds(num_classes: int, world: int, rank: int) -> Tuple[int, int]:
@@ -93,9 +93,10 @@ class ShardedASoftmaxHead:
                  device="cuda", group=None, lambda_state: Optional[LambdaState] = None,
                  weights_full: Optional[torch.Tensor] = None, seed: int = 0, shard_compute=None,
                  transport: str = "nccl", batch_global: Optional[int] = None,
-                 weights_shard: Optional[torch.Tensor] = None, margin: Optional[AdditiveMargin] = None,
+                 weights_shard: Optional[torch.Tensor] = None, margin=None,
                  loss: Optional[FocalLoss] = None):
-        """`margin` (an AdditiveMargin) selects the ArcFace / CosFace head; None: A-softmax.
+        """`margin` (an AdditiveMargin) selects the ArcFace / CosFace head, LinearSoftmax() the plain
+        classifier x_i . w_j; None: A-softmax.
         `loss` (a FocalLoss) replaces the cross-entropy by the focal loss on both transports;
         None: cross-entropy.  An injected `shard_compute` is given the margin and the loss
         through its own constructor."""
